@@ -4,6 +4,7 @@ scene at 1/2/4/8 B200).
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference ...                      (the reference's own CPU implementation on the host cores)
+    python bench.py ... --dump-outputs DIR                    (+ a seeded sample of the last timed step's frames, DIR/*.npy)
 
 A step = one pass of the hot path over one batch of synthetic input = ONE 3840x2160 frame per GPU of the procedural
 512^3 terrain (~32 M voxels, BASELINE.json configs[2]) with the reference CLI's default combination (Voxel Cluster Store +
@@ -180,8 +181,10 @@ def run_reference_arm(args, rank, world):
         ref.render(cams[i], WIDTH, HEIGHT, ALGORITHM, want_hits=False, threads=cores)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        ref.render(cams[args.warmup + i], WIDTH, HEIGHT, ALGORITHM, want_hits=False, threads=cores)
+        last = ref.render(cams[args.warmup + i], WIDTH, HEIGHT, ALGORITHM, want_hits=False, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [last["rgb"]])
     value = WIDTH * HEIGHT * args.steps / dt / 1e6
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -193,6 +196,22 @@ def run_reference_arm(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_PIXELS = 1 << 21     # sampled pixels over all dumped frames: 2^21 x 12 B of colour + 2^21 / frames x 4 B of index <= 32 MiB
+
+
+def dump_outputs(directory, frames):
+    """--dump-outputs: the frames of the last timed step (one per rank, HxWx3 uint8) at a fixed, seeded sample of pixel positions
+    (the same for every frame and every run), as float32 .npy files in `directory`:
+        frame_rgb.npy          (frames, pixels, 3)  colour channels 0..255
+        frame_pixel_index.npy  (pixels,)            row-major pixel index y * WIDTH + x (< 2^24: exact in float32)"""
+    os.makedirs(directory, exist_ok=True)
+    n = DUMP_PIXELS // len(frames)
+    idx = np.sort(np.random.default_rng(20240101).choice(WIDTH * HEIGHT, n, replace=False))
+    rgb = np.stack([np.asarray(f).reshape(WIDTH * HEIGHT, 3)[idx] for f in frames]).astype(np.float32)
+    np.save(os.path.join(directory, "frame_rgb.npy"), rgb)
+    np.save(os.path.join(directory, "frame_pixel_index.npy"), idx.astype(np.float32))
 
 
 def _orbit_args(view):
@@ -256,7 +275,13 @@ def main():
     ap.add_argument("--no-baselines", action="store_true", help="skip the cpu_baseline / ref_gpu / orbit legs (profiling runs)")
     ap.add_argument("--single-view", action="store_true", help="every step renders view 0 (the named single view; profiling runs)")
     ap.add_argument("--orbit-only", action="store_true", help="only the strong-scaling leg (configs[3], the 2048^3 orbit); prints its dict (tuning runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the frames of the last timed step to DIR/*.npy (float32), "
+                                                          "to compare the outputs of two builds run with the same arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.orbit_only:
+        ap.error("--dump-outputs dumps the frames of the timed steps; --orbit-only has none")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -378,6 +403,10 @@ def main():
     tk_ms = float(sum(kern_ms))
     if int(wait_status.item()) != 0:
         raise SystemExit("bench.py: timed out waiting for the completion words of the other ranks")
+    # the frames of the last timed step as rank 0 holds them (copied before later renders reuse `frame`)
+    last_frames = None
+    if args.dump_outputs and rank == 0 and peer is None:
+        last_frames = [frame.cpu()] if world == 1 else [g.cpu() for g in gathered]
 
     exchange_ok = None
     if peer is not None:
@@ -386,6 +415,8 @@ def main():
         dist.barrier()
         if rank == 0:
             full = peer.to_tensor()
+            if args.dump_outputs:
+                last_frames = [full[r * ring + (total - 1) % ring].cpu() for r in range(world)]
             exchange_ok = True
             for r in range(world):
                 for i in (total - 2, total - 1):
@@ -518,6 +549,8 @@ def main():
         if peer is not None:
             peer.close()
         dist.destroy_process_group()
+    if last_frames is not None:
+        dump_outputs(args.dump_outputs, last_frames)
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
     if rank == 0:

@@ -28,6 +28,15 @@ PROBE_CAMERAS = [
 MINI_CAMERAS = [((20.0, 18.0, 26.0), (3.0, 2.0, 0.0), 60.0), ((-30.0, 40.0, -35.0), (3.0, 2.0, 4.0), 60.0)]
 
 
+CONFIG_SAMPLE = 1536    # positions per frame / ray buffer stored in tests/golden/config_golden.npz
+
+
+def config_sample(n):
+    """The fixed, seeded positions (row-major pixels, or rays) of an output of n positions at which tests/golden/config_golden.npz
+    stores the configuration tests' results."""
+    return np.sort(np.random.default_rng(n).choice(n, CONFIG_SAMPLE, replace=False))
+
+
 def oracle_kind():
     """The strongest checker available: the unmodified reference built for the host, else its C restatement."""
     return "refh" if po.available("refh") else "orc"

@@ -76,7 +76,7 @@ def test_empty_scene_renders_background():
     assert not r["rgb"].any() and not r["hits"].any()
 
 
-@pytest.mark.skipif(not po.available("refh"), reason="reference host build not present")
+@pytest.mark.skipif(not po.available("refh"), reason="needs a build of the original project in oracle/_ref (oracle/Makefile, from a reference checkout that is not part of this repository)")
 @pytest.mark.parametrize("storage,algo", COMBOS)
 def test_port_matches_reference_live(storage, algo):
     """Differential run against the unmodified reference: RGB, hit map and per-pixel lookup counts must all agree."""
@@ -99,7 +99,7 @@ def test_port_matches_reference_live(storage, algo):
     assert np.array_equal(ta["colour"], tb["colour"]) and np.array_equal(ta["hits"], tb["hits"])
 
 
-@pytest.mark.skipif(not po.available("refh"), reason="reference host build not present")
+@pytest.mark.skipif(not po.available("refh"), reason="needs a build of the original project in oracle/_ref (oracle/Makefile, from a reference checkout that is not part of this repository)")
 def test_scene_generators_match_reference_generators():
     """scenes.hollow_cube / sphere_shell restate VoxelCube.cuh / VoxelSphere.cuh: compare through the lookup seam."""
     ref = po.OracleScene("refh")
