@@ -100,6 +100,28 @@ int vrm_scene_generate_sparse_shells(vrm_scene* scene, uint32_t size, uint32_t c
 int vrm_scene_generate_cube(vrm_scene* scene, int32_t x, int32_t y, int32_t z, int32_t half_width, uint64_t* n_out);
 int vrm_scene_generate_sphere(vrm_scene* scene, uint32_t x, uint32_t y, uint32_t z, uint32_t radius, int checkered, uint64_t* n_out);
 
+/* ---- dense volumes -------------------------------------------------------------------------------------------------------
+ * LAYOUT (every dense entry point): a volume of dims = {nx, ny, nz} at origin = {ox, oy, oz} is a C-contiguous uint32 array
+ * indexed [x][y][z] -- element (i*ny + j)*nz + k is the voxel at (ox+i, oy+j, oz+k), z fastest; shape (nx, ny, nz) in numpy /
+ * torch.  This is the bit order of a VCS cluster word (x%8 << 6 | y%8 << 3 | z%8), so a z-run of 8 cells shares one occupancy word.
+ * The reference has no counterpart: the nearest are a loop of VoxelSceneCPU::insertVoxel over the cells
+ * (geometry/VoxelSceneCPU.cuh:16-46) and one StorageStructure::lookupVoxel per cell (storage/StorageStructure.cuh:12-17).
+ *
+ * vrm_scene_add_dense[_device]: every cell whose value is not empty_value is appended to the staging list IN LINEAR-INDEX
+ * ORDER, its value as the colour -- exactly what one vrm_scene_add_voxels call with those voxels in that order appends, so
+ * last-insert-wins holds across calls of either kind.  Legal only before vrm_scene_build (VRM_ERR_STATE after).  Every cell of
+ * the box must satisfy |c| < 2^23 and the scene must stay below 2^32 staged voxels (VRM_ERR_INVALID otherwise).  A zero
+ * dimension adds nothing (n_out = 0).  n_out (nullable) receives the number of voxels added.  The compaction runs on the GPU
+ * (count pass, scan, fill pass); it synchronises the handle's stream ONCE to learn the count, then enqueues the fill.
+ *   host variant: the volume travels through a bounded device buffer in slabs of whole x-planes (256 MiB; one synchronisation
+ *                 per slab); the caller may reuse it on return.
+ *   device variant: d_volume must be 4-byte aligned (VRM_ERR_INVALID otherwise); the work is enqueued on the handle's stream and
+ *                 d_volume must stay valid until work ordered after the call on that stream runs (or vrm_scene_synchronize). */
+int vrm_scene_add_dense(vrm_scene* scene, const uint32_t* volume, const uint32_t dims[3], const int32_t origin[3],
+                        uint32_t empty_value, uint64_t* n_out);
+int vrm_scene_add_dense_device(vrm_scene* scene, const uint32_t* d_volume, const uint32_t dims[3], const int32_t origin[3],
+                               uint32_t empty_value, uint64_t* n_out);
+
 /* Build the chosen structure ON THE GPU (radix sort -> last-wins dedupe -> region directory ->
  * VCS cluster tables or cuckoo insertion).  build_ms (nullable) receives the device time. */
 int vrm_scene_build(vrm_scene* scene, int storage_type, float* build_ms);
@@ -214,6 +236,17 @@ int vrm_render_views_sharded(vrm_scene* const* scenes, uint32_t n_scenes, const 
 /* The storage seam on GLOBAL voxel coordinates: out[i] = colour or VRM_EMPTY; exists_out[i] (nullable) =
  * doesVoxelSpaceExist (always 1 inside a non-empty region for the hash table; cluster occupancy for the VCS). */
 int vrm_lookup(vrm_scene* scene, const int32_t* xyz, uint64_t n, uint32_t* out, uint8_t* exists_out);
+
+/* A box of a BUILT scene as a dense volume (layout: "dense volumes" above): out[cell] = exactly what vrm_lookup returns for the
+ * cell's coordinate, the colour or VRM_EMPTY, for both storage types; cells outside the region table or with |c| >= 2^23 read
+ * VRM_EMPTY.  Legal only after vrm_scene_build (VRM_ERR_STATE before); origin + dims must not overflow int32 (VRM_ERR_INVALID);
+ * a zero dimension writes nothing.  The scene scene_box = origin (64 * min_coord)^3, dims (64 * diameter)^3 (vrm_scene_info)
+ * covers every stored voxel.
+ *   host variant: synchronous; the box is read in slabs of whole x-planes through a bounded device buffer (256 MiB), so any box
+ *                 that fits in host memory works.
+ *   device variant: asynchronous on the handle's stream; d_out must be 4-byte aligned (VRM_ERR_INVALID otherwise). */
+int vrm_scene_read_box(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], uint32_t* out);
+int vrm_scene_read_box_device(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], uint32_t* d_out);
 
 /* Opt-in L2 residency hint: an access-policy window (persisting) over the structure's hottest array -- the VCS cluster
  * headers or the hash table's slots -- on the handle's current stream (also VRM_L2_PERSIST=1 at vrm_scene_create).  Off by

@@ -36,6 +36,7 @@ EXPORTS = [
     "vrm_render_device", "vrm_render_views_device", "vrm_render_views_device_strided", "vrm_render_views", "vrm_trace_rays", "vrm_trace_rays_device", "vrm_lookup",
     "vrm_set_l2_persistence", "vrm_set_statistics", "vrm_get_statistics", "vrm_peer_alloc", "vrm_peer_open", "vrm_peer_close", "vrm_peer_free", "vrm_copy_device", "vrm_microbench_l2",
     "vrm_scene_set_completion_flag", "vrm_scene_set_completion_counter", "vrm_claim_next", "vrm_wait_flags_device", "vrm_render_views_sharded",
+    "vrm_scene_add_dense", "vrm_scene_add_dense_device", "vrm_scene_read_box", "vrm_scene_read_box_device",
 ]
 
 
@@ -101,6 +102,10 @@ def load_library():
         "vrm_claim_next": (ci, [ci, vp, vp, vp]),
         "vrm_wait_flags_device": (ci, [ci, vp, vp, u32, u32, u32, u32, vp]),
         "vrm_render_views_sharded": (ci, [vp, u32, vp, u32, vp, u32, ci, u32, u32, vp, ci, vp, C.POINTER(f32)]),
+        "vrm_scene_add_dense": (ci, [vp, vp, vp, vp, u32, C.POINTER(u64)]),
+        "vrm_scene_add_dense_device": (ci, [vp, vp, vp, vp, u32, C.POINTER(u64)]),
+        "vrm_scene_read_box": (ci, [vp, vp, vp, vp]),
+        "vrm_scene_read_box_device": (ci, [vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -133,6 +138,15 @@ def _ptr(a):
 
 def _f3(v):
     return np.ascontiguousarray(np.asarray(v, np.float32).reshape(3))
+
+
+def _box(origin, dims):
+    """(origin, dims) of a dense volume as the int32[3] / uint32[3] arrays of the C ABI."""
+    o = np.ascontiguousarray(np.asarray(origin, np.int64).reshape(3))
+    d = np.ascontiguousarray(np.asarray(dims, np.int64).reshape(3))
+    if (d < 0).any() or (d >= 1 << 32).any() or (o < -(1 << 31)).any() or (o >= 1 << 31).any():
+        raise ValueError(f"box out of range: origin {o.tolist()}, dims {d.tolist()}")
+    return o.astype(np.int32), d.astype(np.uint32)
 
 
 def make_unit_vector(v):
@@ -217,6 +231,46 @@ class VoxelScene:
 
     def add_voxels_device(self, d_xyz_ptr: int, d_rgb_ptr: int, n: int):
         self._check(self.lib.vrm_scene_add_voxels_device(self.h, C.c_void_p(d_xyz_ptr), C.c_void_p(d_rgb_ptr), n), "vrm_scene_add_voxels_device")
+
+    def add_dense(self, volume, origin=(0, 0, 0), empty_value: int = EMPTY) -> int:
+        """Append every cell of ``volume`` (uint32, shape (nx, ny, nz), indexed [x][y][z]: cell [i, j, k] is the voxel at
+        origin + (i, j, k)) whose value is not ``empty_value``, in C order, the value as its colour -- the same list
+        ``add_voxels`` of those voxels in that order would append.  Returns the number of voxels added."""
+        vol = np.asarray(volume)
+        if vol.dtype != np.uint32 or vol.ndim != 3:
+            raise ValueError("add_dense takes a 3-D uint32 volume")
+        vol = np.ascontiguousarray(vol)
+        o, d = _box(origin, vol.shape)
+        n = C.c_uint64()
+        self._check(self.lib.vrm_scene_add_dense(self.h, _ptr(vol), _ptr(d), _ptr(o), int(empty_value), C.byref(n)), "vrm_scene_add_dense")
+        return int(n.value)
+
+    def add_dense_device(self, d_ptr: int, dims, origin=(0, 0, 0), empty_value: int = EMPTY) -> int:
+        """``add_dense`` of a C-contiguous uint32 volume in device memory (4-byte aligned), e.g. ``tensor.data_ptr()``.  Enqueued
+        on the scene's stream after one synchronisation to learn the count; the volume must stay valid until that work has run."""
+        o, d = _box(origin, dims)
+        n = C.c_uint64()
+        self._check(self.lib.vrm_scene_add_dense_device(self.h, C.c_void_p(d_ptr), _ptr(d), _ptr(o), int(empty_value), C.byref(n)),
+                    "vrm_scene_add_dense_device")
+        return int(n.value)
+
+    def read_box(self, origin, dims):
+        """The box ``[origin, origin + dims)`` of the built scene as a uint32 volume of shape ``dims`` (indexed [x][y][z]): the
+        colour of every cell, or ``EMPTY`` -- what ``lookup`` returns for the cell's coordinate."""
+        o, d = _box(origin, dims)
+        out = np.empty(tuple(int(v) for v in d), np.uint32)
+        self._check(self.lib.vrm_scene_read_box(self.h, _ptr(o), _ptr(d), _ptr(out)), "vrm_scene_read_box")
+        return out
+
+    def read_box_device(self, origin, dims, d_out_ptr: int):
+        """``read_box`` into a device buffer of prod(dims) uint32 (4-byte aligned); asynchronous on the scene's stream."""
+        o, d = _box(origin, dims)
+        self._check(self.lib.vrm_scene_read_box_device(self.h, _ptr(o), _ptr(d), C.c_void_p(d_out_ptr)), "vrm_scene_read_box_device")
+
+    def scene_box(self):
+        """(origin, dims) of the box the built scene's region table covers: every stored voxel lies inside it."""
+        info = self.info()
+        return (64 * info["min_coord"],) * 3, (64 * info["diameter"],) * 3
 
     def generate_terrain(self, size: int = 512, seed: int = 1234, max_height: int = 0) -> int:
         """``scenes.terrain(size, seed, max_height)`` generated on the GPU straight into the staging list; returns the voxel count."""
