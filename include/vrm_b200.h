@@ -248,6 +248,31 @@ int vrm_lookup(vrm_scene* scene, const int32_t* xyz, uint64_t n, uint32_t* out, 
 int vrm_scene_read_box(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], uint32_t* out);
 int vrm_scene_read_box_device(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], uint32_t* d_out);
 
+/* ---- voxel lists out -----------------------------------------------------------------------------------------------------
+ * The sparse counterpart of vrm_scene_read_box: every voxel STORED in the built scene whose coordinate lies in the box
+ * [origin, origin + dims), each once, as xyz_out (n x 3 int32) and rgb_out (n x uint32) -- the arrays vrm_scene_add_voxels takes.
+ * The colour is exactly what vrm_lookup returns for the coordinate (after last-insert-wins dedupe).
+ * ORDER: C order of the box, i.e. sorted by increasing (x, y, z), x slowest and z fastest (the layout of the dense entry points), so the
+ * list is the non-VRM_EMPTY cells of vrm_scene_read_box(origin, dims) in linear-index order -- whatever the storage type or hash seeds.
+ * The one difference: a voxel stored with a colour EQUAL to VRM_EMPTY is listed here (read_box cannot show it).
+ * SIZING: n_out is required and always receives the number of voxels in the box.  xyz_out and rgb_out both NULL: count only (VRM_OK);
+ * exactly one of them NULL: VRM_ERR_INVALID; capacity < count: VRM_ERR_INVALID, nothing is written and n_out still holds the count, so
+ * the caller can size its buffers and call again.  The whole scene is the scene_box of vrm_scene_read_box; its count is unique_voxels.
+ * Legal only after vrm_scene_build (VRM_ERR_STATE before); origin + dims must not overflow int32 (VRM_ERR_INVALID); a zero dimension
+ * counts 0 (VRM_OK); boxes partly or wholly outside the region table are legal (nothing is stored there).
+ * The work scales with the voxels of the region-table cells the box touches, not with its cell count (count pass over the cluster
+ * headers / hash slots of those regions, one synchronisation to learn the count, fill pass, radix sort on a key of the position in the
+ * box, write pass).  Device scratch, from the stream-ordered pool: 16 bytes per listed voxel (24 when the box, clipped to the region
+ * table, has more than 2^32 cells) plus ~1 byte per voxel of sort histograms, and 272 bytes per region for the smaller of the
+ * scene's filled regions and the region-table cells the box touches.
+ *   host variant: synchronous; the caller may reuse its buffers on return (the list goes through a device buffer of 16 bytes per voxel).
+ *   device variant: d_xyz_out and d_rgb_out must be 4-byte aligned (VRM_ERR_INVALID otherwise); the handle's stream is synchronised
+ *                 ONCE to learn the count, the rest is enqueued on it: the outputs are ready in stream order. */
+int vrm_scene_read_voxels(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], int32_t* xyz_out, uint32_t* rgb_out,
+                          uint64_t capacity, uint64_t* n_out);
+int vrm_scene_read_voxels_device(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], int32_t* d_xyz_out, uint32_t* d_rgb_out,
+                                 uint64_t capacity, uint64_t* n_out);
+
 /* Opt-in L2 residency hint: an access-policy window (persisting) over the structure's hottest array -- the VCS cluster
  * headers or the hash table's slots -- on the handle's current stream (also VRM_L2_PERSIST=1 at vrm_scene_create).  Off by
  * default: on the BASELINE scenes the touched working set already lives in L1/L2 and the window measured no gain. */

@@ -37,6 +37,7 @@ EXPORTS = [
     "vrm_set_l2_persistence", "vrm_set_statistics", "vrm_get_statistics", "vrm_peer_alloc", "vrm_peer_open", "vrm_peer_close", "vrm_peer_free", "vrm_copy_device", "vrm_microbench_l2",
     "vrm_scene_set_completion_flag", "vrm_scene_set_completion_counter", "vrm_claim_next", "vrm_wait_flags_device", "vrm_render_views_sharded",
     "vrm_scene_add_dense", "vrm_scene_add_dense_device", "vrm_scene_read_box", "vrm_scene_read_box_device",
+    "vrm_scene_read_voxels", "vrm_scene_read_voxels_device",
 ]
 
 
@@ -106,6 +107,8 @@ def load_library():
         "vrm_scene_add_dense_device": (ci, [vp, vp, vp, vp, u32, C.POINTER(u64)]),
         "vrm_scene_read_box": (ci, [vp, vp, vp, vp]),
         "vrm_scene_read_box_device": (ci, [vp, vp, vp, vp]),
+        "vrm_scene_read_voxels": (ci, [vp, vp, vp, vp, vp, u64, C.POINTER(u64)]),
+        "vrm_scene_read_voxels_device": (ci, [vp, vp, vp, vp, vp, u64, C.POINTER(u64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -266,6 +269,44 @@ class VoxelScene:
         """``read_box`` into a device buffer of prod(dims) uint32 (4-byte aligned); asynchronous on the scene's stream."""
         o, d = _box(origin, dims)
         self._check(self.lib.vrm_scene_read_box_device(self.h, _ptr(o), _ptr(d), C.c_void_p(d_out_ptr)), "vrm_scene_read_box_device")
+
+    def _voxel_box(self, origin, dims):
+        if origin is None and dims is None:
+            origin, dims = self.scene_box()
+        elif origin is None or dims is None:
+            raise ValueError("give both origin and dims, or neither (the whole scene_box())")
+        return _box(origin, dims)
+
+    def count_voxels(self, origin=None, dims=None) -> int:
+        """Number of stored voxels in the box ``[origin, origin + dims)`` (default: ``scene_box()``, whose count is ``unique_voxels``)."""
+        o, d = self._voxel_box(origin, dims)
+        n = C.c_uint64()
+        self._check(self.lib.vrm_scene_read_voxels(self.h, _ptr(o), _ptr(d), None, None, 0, C.byref(n)), "vrm_scene_read_voxels")
+        return int(n.value)
+
+    def read_voxels(self, origin=None, dims=None):
+        """The stored voxels of the box ``[origin, origin + dims)`` (default: ``scene_box()``) as ``(xyz int32 (n, 3), rgb uint32 (n,))``
+        sorted by (x, y, z), z fastest: the non-``EMPTY`` cells of ``read_box`` in C order, plus any voxel stored with the colour ``EMPTY``.
+        The same arrays ``add_voxels`` takes, so ``other.add_voxels(*scene.read_voxels())`` rebuilds the scene."""
+        o, d = self._voxel_box(origin, dims)
+        n = self.count_voxels(o, d)
+        xyz = np.empty((n, 3), np.int32)
+        rgb = np.empty(n, np.uint32)
+        got = C.c_uint64()
+        if n:
+            self._check(self.lib.vrm_scene_read_voxels(self.h, _ptr(o), _ptr(d), _ptr(xyz), _ptr(rgb), n, C.byref(got)), "vrm_scene_read_voxels")
+            assert got.value == n
+        return xyz, rgb
+
+    def read_voxels_device(self, origin, dims, d_xyz_ptr: int, d_rgb_ptr: int, capacity: int) -> int:
+        """``read_voxels`` into device buffers of ``capacity`` voxels (n x 3 int32 and n uint32, 4-byte aligned), e.g. torch tensors.
+        Returns the count after one synchronisation; the voxels are written in stream order on the scene's stream.  A capacity below the
+        count raises and writes nothing; ``count_voxels`` sizes the buffers."""
+        o, d = _box(origin, dims)
+        n = C.c_uint64()
+        self._check(self.lib.vrm_scene_read_voxels_device(self.h, _ptr(o), _ptr(d), C.c_void_p(d_xyz_ptr), C.c_void_p(d_rgb_ptr), int(capacity),
+                                                          C.byref(n)), "vrm_scene_read_voxels_device")
+        return int(n.value)
 
     def scene_box(self):
         """(origin, dims) of the box the built scene's region table covers: every stored voxel lies inside it."""

@@ -774,9 +774,9 @@ int vrm_build_structure(vrm_scene* s, int storageType, float* buildMs)
 size_t vrm_scan_scratch_elems(uint64_t n) { return scan_scratch_elems(n); }
 void vrm_exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint64_t n, uint32_t* scratch, cudaStream_t st) { exclusive_scan(in, out, n, scratch, st); }
 
-// The builder's stable LSD radix sort for other callers (vrm_render.cu orders incoherent rays with it): n (32-bit key, 32-bit value)
-// pairs, the low keyBits bits of the key.  `work` holds vrm_sort_work_elems(n, keyBits) uint32.  On return keys / vals point at the
-// sorted pair (the input pair or the partner pair, depending on the number of passes).
+// The builder's stable LSD radix sort for other callers (vrm_render.cu orders incoherent rays with it, vrm_voxels_out.cu puts voxel lists
+// in C order): n (32- or 64-bit key, 32-bit value) pairs, the low keyBits bits of the key.  `work` holds vrm_sort_work_elems(n, keyBits)
+// uint32.  On return keys / vals point at the sorted pair (the input pair or the partner pair, depending on the number of passes).
 size_t vrm_sort_work_elems(uint64_t n, int keyBits)
 {
 	const uint32_t numTiles = (uint32_t)((n + kSortTile - 1) / kSortTile);
@@ -786,9 +786,11 @@ size_t vrm_sort_work_elems(uint64_t n, int keyBits)
 	return (size_t)(histElems + 64 + scan_scratch_elems(histElems));
 }
 
-void vrm_sort_pairs_u32(uint32_t*& keys, uint32_t*& vals, uint32_t* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work, cudaStream_t st)
+// Launches the radix_hist_kernel / radix_scatter_kernel instantiations of build_typed<K>; K = uint32_t or unsigned long long.
+template <class K>
+static void sort_pairs(K*& keys, uint32_t*& vals, K* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work, cudaStream_t st)
 {
-	if (n == 0) return;
+	if (n == 0 || keyBits <= 0) return;
 	const uint32_t numTiles = (uint32_t)((n + kSortTile - 1) / kSortTile);
 	const int passes = (keyBits + kMaxDigitBits - 1) / kMaxDigitBits;
 	const int digitBits = (keyBits + passes - 1) / passes;
@@ -796,15 +798,26 @@ void vrm_sort_pairs_u32(uint32_t*& keys, uint32_t*& vals, uint32_t* keysB, uint3
 	const uint64_t histElems = (uint64_t)(digitMask + 1u) * numTiles;
 	uint32_t* hist = work;
 	uint32_t* scratch = work + ((histElems + 63) & ~(uint64_t)63);
-	uint32_t* kin = keys; uint32_t* kout = keysB;
+	K* kin = keys; K* kout = keysB;
 	uint32_t* vin = vals; uint32_t* vout = valsB;
 	for (int p = 0; p < passes; p++)
 	{
 		const int shift = p * digitBits;
-		radix_hist_kernel<uint32_t><<<numTiles, kThreads, 0, st>>>(kin, n, shift, digitMask, numTiles, hist);
+		radix_hist_kernel<K><<<numTiles, kThreads, 0, st>>>(kin, n, shift, digitMask, numTiles, hist);
 		exclusive_scan(hist, hist, histElems, scratch, st);
-		radix_scatter_kernel<uint32_t><<<numTiles, kThreads, 0, st>>>(kin, vin, n, shift, digitMask, numTiles, hist, kout, vout);
+		radix_scatter_kernel<K><<<numTiles, kThreads, 0, st>>>(kin, vin, n, shift, digitMask, numTiles, hist, kout, vout);
 		std::swap(kin, kout); std::swap(vin, vout);
 	}
 	keys = kin; vals = vin;
+}
+
+void vrm_sort_pairs_u32(uint32_t*& keys, uint32_t*& vals, uint32_t* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work, cudaStream_t st)
+{
+	sort_pairs<uint32_t>(keys, vals, keysB, valsB, n, keyBits, work, st);
+}
+
+void vrm_sort_pairs_u64(unsigned long long*& keys, uint32_t*& vals, unsigned long long* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work,
+                        cudaStream_t st)
+{
+	sort_pairs<unsigned long long>(keys, vals, keysB, valsB, n, keyBits, work, st);
 }

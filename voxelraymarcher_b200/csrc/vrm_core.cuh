@@ -323,6 +323,44 @@ VRM_HD bool hash_cluster_occupied(const uint32_t* clusterMask, uint32_t ri, uint
 	return ((ldg(clusterMask + (ri * 16u + (cid >> 5))) >> (cid & 31u)) & 1u) != 0u;
 }
 
+// ---- reading the stored voxels back (vrm_voxels_out.cu): the inverses of the two layouts ----
+// hash_key inverse: region-local x, y, z of a stored key
+VRM_HD void hash_key_decode(uint32_t key, uint32_t& x, uint32_t& y, uint32_t& z)
+{
+	constexpr uint32_t m = (1u << kHashKeyBits) - 1u;
+	x = key >> (2 * kHashKeyBits); y = (key >> kHashKeyBits) & m; z = key & m;
+}
+// A hash slot holds (hash_key << 32) | colour, or kEmptySlot.  A region's slots are table 1 and table 2 back to back:
+// [base1, base1 + 2n) of SceneView::slots (load_region below), and after the build every one is a stored voxel of the region or free.
+VRM_HD bool slot_used(unsigned long long e) { return e != kEmptySlot; }
+VRM_HD uint32_t slot_key(unsigned long long e) { return (uint32_t)(e >> 32); }
+VRM_HD uint32_t slot_colour(unsigned long long e) { return (uint32_t)e; }
+// VCS: cluster (cx, cy, cz) of a region (cluster coordinates 0..7) -> cluster id, bit of the region's 512-bit cluster mask
+VRM_HD uint32_t vcs_cluster_id(uint32_t cx, uint32_t cy, uint32_t cz) { return (cx << 6) | (cy << 3) | cz; }
+// header word w (0..15) of cluster cid of dense region ri
+VRM_HD size_t vcs_header_index(uint32_t ri, uint32_t cid, uint32_t w) { return ((size_t)ri * 512 + cid) * 16 + w; }
+// Header word w covers the in-cluster codes 32w .. 32w + 31 (code = x%8 << 6 | y%8 << 3 | z%8): x%8 = w >> 1, y%8 = (w & 1) * 4 + bit / 8,
+// z%8 = bit % 8 -- a z-range is a byte mask, a y-range selects bytes, an x-range selects word pairs.  Mask of the bits of word w whose
+// voxel lies in the cluster-local box [x0, x1) x [y0, y1) x [z0, z1) (0 <= lo < hi <= 8 per axis).
+VRM_HD uint32_t vcs_word_box_mask(uint32_t w, uint32_t x0, uint32_t x1, uint32_t y0, uint32_t y1, uint32_t z0, uint32_t z1)
+{
+	const uint32_t x = w >> 1, yb = (w & 1u) * 4u;
+	if (x < x0 || x >= x1) return 0u;
+	const uint32_t zb = (0xFFu << z0) & ~(0xFFu << z1) & 0xFFu;
+	// bytes b = 0..3 hold y = yb + b: keep those with y0 <= y < y1
+	const uint32_t bLo = y0 > yb ? y0 - yb : 0u, bHi = y1 > yb ? (y1 - yb < 4u ? y1 - yb : 4u) : 0u;
+	if (bLo >= bHi) return 0u;
+	const uint32_t bytes = (0xFFFFFFFFu >> (32u - 8u * (bHi - bLo))) << (8u * bLo);
+	return (zb * 0x01010101u) & bytes;
+}
+// in-cluster coordinates of bit `bit` of header word w
+VRM_HD void vcs_word_bit_xyz(uint32_t w, uint32_t bit, uint32_t& x, uint32_t& y, uint32_t& z)
+{
+	x = w >> 1; y = (w & 1u) * 4u + (bit >> 3); z = bit & 7u;
+}
+// index into SceneView::values of the colour behind a SET bit of a header word {occupancy mask, index of the word's first colour}
+VRM_HD uint32_t vcs_colour_index(uint32_t hx, uint32_t hy, uint32_t bit) { return (hy & ~kHeaderClusterExists) + popc32(hx & ((1u << bit) - 1u)); }
+
 template <int ST> struct RegionRef;
 
 template <> struct RegionRef<kStorageHash>

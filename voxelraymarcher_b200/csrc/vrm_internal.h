@@ -136,9 +136,11 @@ void vrm_free_async(vrm_scene* s, void* p);
 void vrm_configure_pool(int device);
 size_t vrm_scan_scratch_elems(uint64_t n);  // uint32 elements of scratch an exclusive scan of n elements needs
 void vrm_exclusive_scan_u32(const uint32_t* in, uint32_t* out, uint64_t n, uint32_t* scratch, cudaStream_t st);  // out may alias in
-// the builder's stable LSD radix sort on (32-bit key, 32-bit value) pairs (vrm_build.cu)
+// the builder's stable LSD radix sort on (32- or 64-bit key, 32-bit value) pairs (vrm_build.cu)
 size_t vrm_sort_work_elems(uint64_t n, int keyBits);
 void vrm_sort_pairs_u32(uint32_t*& keys, uint32_t*& vals, uint32_t* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work, cudaStream_t st);
+void vrm_sort_pairs_u64(unsigned long long*& keys, uint32_t*& vals, unsigned long long* keysB, uint32_t* valsB, uint64_t n, int keyBits, uint32_t* work,
+                        cudaStream_t st);
 
 // vrm_api.cu: install / remove the access-policy window on the handle's current stream (called by the launch wrappers)
 void vrm_apply_l2_window(vrm_scene* s);
