@@ -571,8 +571,8 @@ __global__ void __launch_bounds__(kShadowThreads, (ALGO == kAlgoOriginal ? 6 : V
 
 // ---- persistent-thread ray queue + warp-level state scheduling ------------------------------------------------------
 // Pixel slots are numbered tile-major: slot = (view * tilesPerView + tile) * 32 + pixel-in-8x4-tile, so that 32 consecutive
-// slots are one warp-coherent tile.  Every lane owns one FlatRay state machine (vrm_flat.cuh).  Per iteration the warp
-// votes (__match_any_sync groups lanes by state, __reduce_min_sync picks the largest group) and runs ONLY that state's
+// slots are one warp-coherent tile.  The tiles are those of the launch's band, rows [yBase, yEnd), as in the grid kernels.
+// Every lane owns one FlatRay state machine (vrm_flat.cuh).  Per iteration the warp votes (__match_any_sync groups lanes by state, __reduce_min_sync picks the largest group) and runs ONLY that state's
 // code block; lanes in other states wait for their turn, lanes whose pixel is resolved vote for a refill, which claims the
 // next slots with one warp-aggregated atomicAdd.  Divergent ray lengths and phases therefore cost idle lanes only while a
 // state is in the minority, instead of serialising every loop nest as the nested kernels do.
@@ -625,8 +625,8 @@ __global__ void __launch_bounds__(kPersistThreads) render_scheduled_kernel(const
 					const unsigned tile = slot >> 5, inTile = slot & 31u;
 					const unsigned view = tile / a.tilesPerView, t = tile - view * a.tilesPerView;
 					const uint32_t x = (t % a.tilesX) * kTileW + (inTile & (kTileW - 1));
-					const uint32_t y = (t / a.tilesX) * kTileH + (inTile / kTileW);
-					if (x < a.W && y < a.H)
+					const uint32_t y = a.yBase + (t / a.tilesX) * kTileH + (inTile / kTileW);
+					if (x < a.W && y < a.yEnd)
 					{
 						const float* cam = a.cams + (size_t)view * 15;
 						float camv[15];
@@ -1277,7 +1277,7 @@ int vrm_launch_render(vrm_scene* s, const float* d_cams, uint32_t nViews, const 
 	a.rowWordsOk = ((W * 3u) % 4u == 0 && (reinterpret_cast<uintptr_t>(d_rgb) & 3u) == 0 && (((size_t)W * H * 3) % 4 == 0 || nViews == 1)) ? 1u : 0u;
 	a.queue = s->d_queue;
 	a.tilesX = (W + kTileW - 1) / kTileW;
-	a.tilesPerView = a.tilesX * ((H + kTileH - 1) / kTileH);
+	a.tilesPerView = a.tilesX * ((yEnd - yBase + kTileH - 1) / kTileH);  // the band's tiles (persistent kernel only)
 	a.nViews = nViews;
 	// 32-bit pixel-slot numbers exist only in the persistent debug kernel (VRM_RENDER_MODE=0); the tiled kernels index with size_t
 	if (s->renderMode == 0 && (uint64_t)a.tilesPerView * nViews * 32ull >= (1ull << 32)) { s->lastError = "too many pixels for one launch of the persistent kernel"; return VRM_ERR_INVALID; }
