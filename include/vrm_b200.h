@@ -123,7 +123,15 @@ int vrm_scene_add_dense_device(vrm_scene* scene, const uint32_t* d_volume, const
                                uint32_t empty_value, uint64_t* n_out);
 
 /* Build the chosen structure ON THE GPU (radix sort -> last-wins dedupe -> region directory ->
- * VCS cluster tables or cuckoo insertion).  build_ms (nullable) receives the device time. */
+ * VCS cluster tables or cuckoo insertion).  build_ms (nullable) receives the device time.
+ * Extent: the cubic region table spans one range of region indices for all three axes and always contains region 0, so
+ * max(0, floor(c_max / 64)) - min(0, floor(c_min / 64)) < 1024 must hold, with c_min and c_max taken over every coordinate of every
+ * staged voxel (e.g. up to 65535 when no coordinate is negative, down to -65472 when none is above 63) -- stricter than the
+ * |c| < 2^23 of vrm_scene_add_voxels.  A wider scene fails with VRM_ERR_INVALID before the staged voxels are touched.
+ * A build that returns an error leaves the handle as if it had not been attempted: the same staged scene (possibly already
+ * deduplicated), so voxels added later still win and a retry -- e.g. VRM_STORAGE_HASHTABLE after the VCS index widths were
+ * exceeded -- builds that scene.  If the staged voxels cannot be restored (an allocation of 12 bytes per voxel fails, or a
+ * CUDA error), they are dropped and every later staging call and vrm_scene_build returns VRM_ERR_STATE. */
 int vrm_scene_build(vrm_scene* scene, int storage_type, float* build_ms);
 
 /* diameter^3 = size of the cubic region table, min_coord = lowest region index on any axis (both as in the

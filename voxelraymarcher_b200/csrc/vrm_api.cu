@@ -256,7 +256,7 @@ int vrm_scene_synchronize(vrm_scene* s)
 static int add_voxels(vrm_scene* s, const int32_t* xyz, const uint32_t* rgb, uint64_t n, bool fromDevice)
 {
 	if (!s || (n && (!xyz || !rgb))) return VRM_ERR_INVALID;
-	if (s->storage >= 0) { s->lastError = "scene already built"; return VRM_ERR_STATE; }
+	if (int rc = vrm_check_staging(s)) return rc;
 	if (n == 0) return VRM_OK;
 	if (!fromDevice && n <= kPendingMaxCall)
 	{
@@ -307,7 +307,7 @@ int vrm_scene_insert_voxel(vrm_scene* s, int32_t x, int32_t y, int32_t z, uint32
 int vrm_scene_build(vrm_scene* s, int storage_type, float* build_ms)
 {
 	if (!s || (storage_type != VRM_STORAGE_VCS && storage_type != VRM_STORAGE_HASHTABLE)) return VRM_ERR_INVALID;
-	if (s->storage >= 0) { s->lastError = "scene already built"; return VRM_ERR_STATE; }
+	if (int rc = vrm_check_staging(s)) return rc;
 	VRM_CUDA(s, cudaSetDevice(s->device));
 	int rc = vrm_build_structure(s, storage_type, build_ms);
 	if (rc == VRM_OK)

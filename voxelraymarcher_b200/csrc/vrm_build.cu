@@ -428,6 +428,65 @@ __global__ void cuckoo_round_end_kernel(unsigned long long* __restrict__ slots, 
 
 unsigned grid_for(uint64_t n) { return (unsigned)((n + kThreads - 1) / kThreads); }
 
+// ---- a failed build gives its voxels back --------------------------------------------------------------------------
+// Inverse of make_keys_kernel: the voxel of a key of the region table (D, minCoord).
+template <class K>
+__global__ void key_to_xyz_kernel(const K* __restrict__ keys, uint64_t n, int minCoord, uint32_t D, int32_t* __restrict__ xyz)
+{
+	uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const K k = keys[i];
+	const uint64_t region = (uint64_t)(k >> 18);
+	const int rx = (int)(region % D) + minCoord, ry = (int)(region / D % D) + minCoord, rz = (int)(region / D / D) + minCoord;
+	const uint32_t cid = (uint32_t)(k >> 9) & 511u, code = (uint32_t)k & 511u;
+	xyz[3 * i] = rx * 64 + (int)(((cid >> 6) << 3) | (code >> 6));
+	xyz[3 * i + 1] = ry * 64 + (int)((((cid >> 3) & 7u) << 3) | ((code >> 3) & 7u));
+	xyz[3 * i + 2] = rz * 64 + (int)(((cid & 7u) << 3) | (code & 7u));
+}
+
+// After the sort the staging list is gone: the colours were sorted in place of d_stageRgb and, with 32-bit keys, the sort's partner
+// buffers were carved out of d_stageXyz.  A build that fails after that point puts n sorted pairs back as the staged list -- the
+// stable-sorted ones (their order keeps last-insert-wins) or the deduplicated ones -- so that the handle stages the same scene as
+// before the build.  The keys may live inside d_stageXyz, so they are decoded into a fresh array.  If even that fails, the staging
+// is marked lost: later staging and build calls return VRM_ERR_STATE instead of building another scene.
+template <class K>
+void restage(vrm_scene* s, const K* keys, const uint32_t* vals, uint64_t n, int minCoord, uint32_t D)
+{
+	int32_t* xyz = nullptr;
+	cudaError_t e = vrm_alloc_async(s, reinterpret_cast<void**>(&xyz), n * 12);
+	if (e == cudaSuccess)
+	{
+		key_to_xyz_kernel<K><<<grid_for(n), kThreads, 0, s->stream>>>(keys, n, minCoord, D, xyz);
+		e = cudaGetLastError();
+	}
+	if (e == cudaSuccess && vals != s->d_stageRgb) e = cudaMemcpyAsync(s->d_stageRgb, vals, n * 4, cudaMemcpyDeviceToDevice, s->stream);
+	if (e != cudaSuccess)
+	{
+		cudaGetLastError();
+		vrm_free_async(s, xyz);
+		vrm_stage_free(s);
+		s->nStaged = 0;
+		s->stageLost = true;
+		s->lastError += " (the staged voxels could not be restored)";
+		return;
+	}
+	vrm_free_async(s, s->d_stageXyz);
+	s->d_stageXyz = xyz;
+	s->stageCap = n;  // d_stageRgb holds at least n
+	s->nStaged = n;
+}
+
+// Armed (keys set) once the sort has consumed the staging list; a return while armed hands the pairs back.  Declared after the
+// buffers that hold them, so it runs before their stream-ordered frees.
+template <class K>
+struct RestageOnFailure
+{
+	vrm_scene* s; int minCoord; uint32_t D;
+	const K* keys = nullptr; const uint32_t* vals = nullptr; uint64_t n = 0;
+	void arm(const K* k, const uint32_t* v, uint64_t count) { keys = k; vals = v; n = count; }
+	~RestageOnFailure() { if (keys) restage(s, keys, vals, n, minCoord, D); }
+};
+
 // VRM_BUILD_TRACE=1: host-clock stage marks on stderr (each mark synchronises the stream, so traced builds are slower)
 struct BuildTrace
 {
@@ -459,6 +518,7 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 	uint64_t unique = 0;
 	uint32_t numRegions = 0;
 	PoolBuf keysA(s), extra(s), uniq(s), regionStart(s), cellBuf(s);
+	RestageOnFailure<K> restore{s, minCoord, (uint32_t)D};
 	K* ukeys = nullptr;
 	uint32_t* uvals = nullptr;
 	bool valsAreStageRgb = false;  // uvals == s->d_stageRgb: the colour array can change owner without a copy
@@ -499,6 +559,7 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 			radix_scatter_kernel<K><<<numTiles, kThreads, 0, st>>>(kin, vin, n, shift, digitMask, numTiles, hist, kout, vout);
 			std::swap(kin, kout); std::swap(vin, vout);
 		}
+		restore.arm(kin, vin, n);
 		trace.mark(st, "radix sort");
 		// ---- 3. + 4. dedupe flags, region heads, one read-back of {unique, regions} (kout / vout are free now) ------------
 		uint32_t* keep = vout;
@@ -527,6 +588,7 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 			ukeys = uniq.as<K>();
 			uvals = reinterpret_cast<uint32_t*>(uniq.as<char>() + pad256(unique * sizeof(K)));
 			compact_kernel<K><<<grid_for(n), kThreads, 0, st>>>(kin, vin, keep, pos, n, ukeys, uvals);
+			restore.arm(ukeys, uvals, unique);
 		}
 		trace.mark(st, "dedupe + region heads");
 		if (regionStart.alloc(((size_t)numRegions + 1) * 4) != cudaSuccess) { cudaGetLastError(); s->lastError = "region directory allocation failed"; return VRM_ERR_NOMEM; }
@@ -557,9 +619,9 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 			vcs_fill_kernel<K><<<grid_for(unique), kThreads, 0, st>>>(ukeys, regionTable.as<int32_t>(), unique, headers.as<uint2>(), clusterMask.as<uint32_t>());
 			vcs_flag_clusters_kernel<<<grid_for((uint64_t)numRegions * 512), kThreads, 0, st>>>(headers.as<uint2>(), clusterMask.as<uint32_t>(), (uint64_t)numRegions * 512);
 		}
-		// the colours outlive the build: the staging array itself when the sort ended there, else one device copy
-		if (unique && valsAreStageRgb) { values.s = s; values.p = s->d_stageRgb; s->d_stageRgb = nullptr; }
-		else
+		// the colours outlive the build: the staging array itself when the sort ended there (it changes owner once nothing can fail any
+		// more, below), else one device copy
+		if (!(unique && valsAreStageRgb))
 		{
 			if (values.alloc(unique * 4) != cudaSuccess) { cudaGetLastError(); s->lastError = "colour array allocation failed"; return VRM_ERR_NOMEM; }
 			if (unique) VRM_CUDA(s, cudaMemcpyAsync(values.p, uvals, unique * 4, cudaMemcpyDeviceToDevice, st));
@@ -625,7 +687,8 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 	{
 		s->d_headers = static_cast<uint2*>(headers.release());
 		s->d_clusterMask = static_cast<uint32_t*>(clusterMask.release());
-		s->d_values = static_cast<uint32_t*>(values.release());
+		if (unique && valsAreStageRgb) { s->d_values = s->d_stageRgb; s->d_stageRgb = nullptr; }
+		else s->d_values = static_cast<uint32_t*>(values.release());
 	}
 	else
 	{
@@ -639,6 +702,7 @@ int build_typed(vrm_scene* s, int storageType, int keyBits, int minCoord, uint64
 	s->filled = numRegions;
 	s->unique = unique;
 	s->bytes = bytes;
+	restore.keys = nullptr;
 	return VRM_OK;
 }
 

@@ -171,7 +171,7 @@ int add_dense(vrm_scene* s, const uint32_t* volume, const uint32_t* dims, const 
 {
 	if (n_out) *n_out = 0;
 	if (!s || !dims || !origin) return VRM_ERR_INVALID;
-	if (s->storage >= 0) { s->lastError = "scene already built"; return VRM_ERR_STATE; }
+	if (int rc = vrm_check_staging(s)) return rc;
 	if (dims[0] == 0 || dims[1] == 0 || dims[2] == 0) return VRM_OK;
 	if (!volume) { s->lastError = "volume is NULL"; return VRM_ERR_INVALID; }
 	if (fromDevice && (reinterpret_cast<uintptr_t>(volume) & 3u)) { s->lastError = "device volume must be 4-byte aligned"; return VRM_ERR_INVALID; }

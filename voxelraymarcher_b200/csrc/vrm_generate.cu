@@ -221,7 +221,7 @@ int scan_counts(vrm_scene* s, const uint32_t* counts, uint32_t* starts, uint64_t
 int check_generate(vrm_scene* s)
 {
 	if (!s) return VRM_ERR_INVALID;
-	if (s->storage >= 0) { s->lastError = "scene already built"; return VRM_ERR_STATE; }
+	if (int rc = vrm_check_staging(s)) return rc;
 	VRM_CUDA(s, cudaSetDevice(s->device));
 	return VRM_OK;
 }

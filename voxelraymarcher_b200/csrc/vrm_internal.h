@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "vrm_core.cuh"
+#include "../../include/vrm_b200.h"
 
 // Small inserts (vrm_scene_insert_voxel, short vrm_scene_add_voxels calls) are collected on the host and reach the device in
 // blocks of this many voxels: a caller porting the reference's insertVoxel loop (VoxelSceneCPU.cuh:16-46) pays a vector append per
@@ -30,6 +31,7 @@ struct vrm_scene
 	// ... behind a host-side block of voxels that have not been copied yet (kPendingFlushVoxels)
 	std::vector<int32_t> pendingXyz;
 	std::vector<uint32_t> pendingRgb;
+	bool stageLost = false;          // a failed build could not restore the staged voxels (vrm_build.cu restage): no more staging or builds
 
 	// built structure
 	int storage = -1;
@@ -118,6 +120,14 @@ int vrm_fail_cuda(vrm_scene* s, cudaError_t e, const char* what);
 		cudaError_t e__ = (call);                                           \
 		if (e__ != cudaSuccess) return vrm_fail_cuda((s), e__, #call);      \
 	} while (0)
+
+// The staging calls and vrm_scene_build are legal only before a build and while the staged voxels exist.
+inline int vrm_check_staging(vrm_scene* s)
+{
+	if (s->storage >= 0) { s->lastError = "scene already built"; return VRM_ERR_STATE; }
+	if (s->stageLost) { s->lastError = "the staged voxels were lost when a build failed; create a new scene"; return VRM_ERR_STATE; }
+	return VRM_OK;
+}
 
 // vrm_build.cu
 int vrm_build_structure(vrm_scene* s, int storageType, float* buildMs);
