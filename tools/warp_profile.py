@@ -3,6 +3,10 @@ march_scene_flat_warp on the CPU (tests/hostsim: the product's own traversal sou
 bench frame (512^3 terrain, 3840x2160, view 0), VCS + longest axis.
 
     python tools/warp_profile.py [--size 512] [--stride 4] [--view 0]
+    python tools/warp_profile.py --views 20 --horizon both   # passes per tile over bench.py's view sequence, shadow horizon map off / on
+
+The library is tests/horizon_sim.py's host build (tests/hostsim plus the horizon map's entry points); terrain cameras are made there with
+Camera.cuh's formula, as api.Camera, so the tool needs no GPU library.
 """
 import argparse
 import ctypes
@@ -13,10 +17,19 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from voxelraymarcher_b200 import api, scenes  # noqa: E402
+from voxelraymarcher_b200 import scenes  # noqa: E402
+from tests import horizon_sim  # noqa: E402
 import bench  # noqa: E402
 
 CATS = ["region", "head", "test", "jump", "next", "cluster", "nullreg", "hitwait", "done"]
+
+
+def camera(lib, view):
+    org, at, up, fov, aspect = bench._orbit_args(view)
+    out = np.zeros(15, np.float32)
+    f3 = [np.ascontiguousarray(v, np.float32) for v in (org, at, up)]
+    lib.hz_camera_make(*(v.ctypes.data_as(ctypes.c_void_p) for v in f3), ctypes.c_float(fov), ctypes.c_float(aspect), out.ctypes.data_as(ctypes.c_void_p))
+    return out
 
 
 def main():
@@ -28,9 +41,10 @@ def main():
     ap.add_argument("--regroup", default="", help="budget:maxLanes[,budget:maxLanes...]: simulate abandon + re-trace of long-tailed tiles (sim_regroup_profile)")
     ap.add_argument("--compact", default="", help="tiles per CTA, e.g. 2,4,8: simulate packing the shadow rays of a CTA's tiles into full warps (sim_cta_compact_profile)")
     ap.add_argument("--scene", default="terrain", choices=["terrain", "shells2048"], help="shells2048: BASELINE configs[3], one 1080p view of its orbit")
+    ap.add_argument("--horizon", default="off", choices=["off", "on", "both"], help="--views: shadow rays end at the horizon map (vrm_core.cuh HorizonView)")
+    ap.add_argument("--views", type=int, default=0, help="terrain: passes per tile over the first N views of bench.py's sequence (bench.view_of) instead of one profile")
     a = ap.parse_args()
-    lib = ctypes.CDLL(os.path.join(ROOT, "tests", "hostsim", "libhostsim.so"))
-    lib.sim_scene_create.restype = ctypes.c_void_p
+    lib = horizon_sim.load()
     if a.scene == "terrain":
         xyz, rgb = scenes.terrain(a.size, bench.SCENE_SEED)
     else:
@@ -44,12 +58,31 @@ def main():
     lib.sim_make_unit_vector(np.array([1.0, 1.0, 1.0], np.float32).ctypes.data_as(ctypes.c_void_p), d.ctypes.data_as(ctypes.c_void_p))
     W, H = bench.WIDTH, bench.HEIGHT
     if a.scene == "terrain":
-        cam = bench.orbit_camera(api, a.view)
+        camv = camera(lib, a.view)
     else:
+        from voxelraymarcher_b200 import api
         W, H = 1920, 1080
-        cam = bench.orbit_views_2048(api, W, H)[a.view]
-    camv = np.ascontiguousarray(cam.data, np.float32)
+        camv = np.ascontiguousarray(bench.orbit_views_2048(api, W, H)[a.view].data, np.float32)
     tr = np.zeros(3, np.float32)
+    if a.views:
+        views = [bench.view_of(k, 0, 1) for k in range(a.views)]
+        modes = [0, 1] if a.horizon == "both" else [int(a.horizon == "on")]
+        per = {}
+        for m in modes:
+            for v in views:
+                cv = camera(lib, v)
+                tot = np.zeros(3, np.uint64)
+                assert lib.hz_warp_passes(h, cv.ctypes.data_as(ctypes.c_void_p), tr.ctypes.data_as(ctypes.c_void_p), 1, W, H, a.stride, m,
+                                          tot.ctypes.data_as(ctypes.c_void_p), a.threads) == 0
+                per[(m, v)] = (int(tot[1]) / int(tot[0]), int(tot[2]) / int(tot[0]))
+                print(f"horizon {'on ' if m else 'off'} view {v:2d}: passes/tile {per[(m, v)][0]:6.2f} (shadow {per[(m, v)][1]:6.2f})", flush=True)
+        for m in modes:
+            p = np.mean([per[(m, v)][0] for v in views]); sp = np.mean([per[(m, v)][1] for v in views])
+            print(f"horizon {'on ' if m else 'off'}: mean over {len(views)} views: passes/tile {p:.3f}, shadow passes/tile {sp:.3f}")
+        if len(modes) == 2:
+            off = np.mean([per[(0, v)][0] for v in views]); on = np.mean([per[(1, v)][0] for v in views])
+            print(f"passes per tile: {100 * (off - on) / off:.1f} % fewer with the horizon map")
+        return
     if a.compact:
         for tpc in (int(v) for v in a.compact.split(",")):
             out = np.zeros(7, np.uint64)

@@ -190,6 +190,7 @@ int vrm_scene_create(int device, vrm_scene** out)
 	if (const char* ws = getenv("VRM_WSTORE_REMOTE")) s->wstoreRemote = atoi(ws) != 0;
 	if (const char* bs = getenv("VRM_BULK_STORE")) s->bulkStore = atoi(bs) != 0;
 	if (const char* bb = getenv("VRM_VIEW_BATCH_BYTES")) { long long v = atoll(bb); if (v > 0) s->viewBatchBytes = (size_t)v; }
+	if (const char* sh = getenv("VRM_SHADOW_HORIZON")) s->horizonEnabled = atoi(sh) != 0;
 	if (e != cudaSuccess) { vrm_scene_destroy(s); cudaGetLastError(); return VRM_ERR_CUDA; }
 	s->stream = s->ownStream;
 	cudaEventRecord(s->ev1, s->stream);
@@ -206,7 +207,7 @@ int vrm_scene_destroy(vrm_scene* s)
 	vrm_free_async(s, s->d_regionMinMax); s->d_regionMinMax = nullptr;
 	vrm_free_structure(s);
 	cudaStreamSynchronize(s->stream);
-	cudaFree(s->d_hits); cudaFree(s->d_cams); cudaFree(s->d_io); cudaFree(s->d_stats); cudaFree(s->d_queue); cudaFree(s->d_defer); cudaFree(s->d_parkBits); cudaFree(s->d_parkCtl); cudaFree(s->d_gather); cudaFree(s->d_shadowItems); cudaFree(s->d_shadowCtl); cudaFree(s->d_localFrame); if (s->h_stage) cudaFreeHost(s->h_stage); for (auto& e : s->evBand) if (e) cudaEventDestroy(e);
+	cudaFree(s->d_hits); cudaFree(s->d_cams); cudaFree(s->d_io); cudaFree(s->d_stats); cudaFree(s->d_queue); cudaFree(s->d_defer); cudaFree(s->d_parkBits); cudaFree(s->d_parkCtl); cudaFree(s->d_gather); cudaFree(s->d_shadowItems); cudaFree(s->d_shadowCtl); cudaFree(s->d_localFrame); vrm_free_async(s, s->d_horizon); cudaStreamSynchronize(s->stream); if (s->h_stage) cudaFreeHost(s->h_stage); for (auto& e : s->evBand) if (e) cudaEventDestroy(e);
 	if (s->h_cams) cudaFreeHost(s->h_cams);
 	if (s->ev0) cudaEventDestroy(s->ev0);
 	if (s->ev1) cudaEventDestroy(s->ev1);
@@ -334,8 +335,15 @@ int vrm_scene_info(const vrm_scene* s, uint32_t* diameter, int32_t* min_coord, u
 int vrm_set_lighting(vrm_scene* s, const float direction[3], const float colour[3], const float position[3], int use_point_light, int use_shadows)
 {
 	if (!s || !direction || !colour || !position) return VRM_ERR_INVALID;
+	const bool newMap = memcmp(s->light.dir, direction, 12) != 0 || (s->light.useShadows != 0) != (use_shadows != 0);
 	memcpy(s->light.dir, direction, 12); memcpy(s->light.color, colour, 12); memcpy(s->light.pos, position, 12);
 	s->light.usePoint = use_point_light != 0; s->light.useShadows = use_shadows != 0;
+	if (newMap && s->storage >= 0)
+	{
+		// the shadow horizon map belongs to the light direction: rebuilt on the handle's stream, behind the launches that still read the old one
+		VRM_CUDA(s, cudaSetDevice(s->device));
+		return vrm_build_horizon(s);
+	}
 	return VRM_OK;
 }
 

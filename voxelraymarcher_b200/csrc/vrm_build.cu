@@ -807,6 +807,55 @@ void vrm_free_structure(vrm_scene* s)
 	s->storage = -1; s->bytes = 0; s->filled = 0; s->unique = 0;
 }
 
+// ---- shadow horizon map (vrm_core.cuh HorizonView) --------------------------------------------------------------------------------
+// One thread per (region-table entry, 32-cluster word of its cluster-exists mask), grid-stride: each occupied cluster of the word
+// max-es its depth bound into the cells its widened projection covers.
+__global__ void horizon_kernel(HorizonView h, int32_t* __restrict__ cells, const int32_t* __restrict__ regionTable, const uint32_t* __restrict__ clusterMask,
+                               uint32_t D)
+{
+	const unsigned long long total = (unsigned long long)D * D * D * 16ull;
+	for (unsigned long long t = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; t < total; t += (unsigned long long)gridDim.x * blockDim.x)
+	{
+		const unsigned long long e = t >> 4;
+		const int32_t ri = __ldg(regionTable + e);
+		if (ri < 0) continue;
+		const uint32_t w = (uint32_t)(t & 15u);
+		uint32_t bits = __ldg(clusterMask + (size_t)ri * 16u + w);
+		const uint32_t ux = (uint32_t)(e % D), uy = (uint32_t)((e / D) % D), uz = (uint32_t)(e / ((unsigned long long)D * D));
+		while (bits)
+		{
+			const uint32_t cid = w * 32u + (uint32_t)(__ffs(bits) - 1);
+			bits &= bits - 1u;
+			horizon_splat(h, ux * 8u + (cid >> 6), uy * 8u + ((cid >> 3) & 7u), uz * 8u + (cid & 7u), [&](uint32_t i, int32_t v) { atomicMax(cells + i, v); });
+		}
+	}
+}
+
+int vrm_build_horizon(vrm_scene* s)
+{
+	s->horizon.cells = nullptr;
+	// only the VCS + longest-axis state machine reads the map (vrm_render.cu: fused render and trace kernels)
+	if (!s->horizonEnabled || s->storage != VRM_STORAGE_VCS || !s->light.useShadows) return VRM_OK;
+	const PermRuntime p = rank_axes(s->light.dir[0], s->light.dir[1], s->light.dir[2]);
+	HorizonView h;
+	if (!horizon_setup(s->light.dir, s->diameter, (uint32_t)p.a0, h)) return VRM_OK;
+	const size_t n = (size_t)h.nu * h.nv;
+	if (s->horizonCap < n)
+	{
+		vrm_free_async(s, s->d_horizon); s->d_horizon = nullptr; s->horizonCap = 0;
+		VRM_CUDA(s, vrm_alloc_async(s, reinterpret_cast<void**>(&s->d_horizon), n * sizeof(int32_t)));
+		s->horizonCap = n;
+	}
+	VRM_CUDA(s, cudaMemsetAsync(s->d_horizon, 0x80, n * sizeof(int32_t), s->stream));  // kHorizonEmpty
+	const unsigned long long work = (unsigned long long)s->diameter * s->diameter * s->diameter * 16ull;
+	const unsigned blocks = (unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)s->numSms * 32ull);
+	horizon_kernel<<<blocks, 256, 0, s->stream>>>(h, s->d_horizon, s->d_regionTable, s->d_clusterMask, s->diameter);
+	VRM_CUDA(s, cudaGetLastError());
+	h.cells = s->d_horizon;
+	s->horizon = h;
+	return VRM_OK;
+}
+
 int vrm_build_structure(vrm_scene* s, int storageType, float* buildMs)
 {
 	cudaStream_t st = s->stream;
@@ -830,6 +879,12 @@ int vrm_build_structure(vrm_scene* s, int storageType, float* buildMs)
 	const int keyBits = 18 + regionBits;
 	rc = keyBits <= 32 ? build_typed<uint32_t>(s, storageType, keyBits, minCoord, D, trace) : build_typed<unsigned long long>(s, storageType, keyBits, minCoord, D, trace);
 	if (rc) return rc;
+	// the shadow horizon map is part of the build (and of its time)
+	rc = vrm_build_horizon(s);
+	if (rc) return rc;
+	VRM_CUDA(s, cudaEventRecord(s->ev1, st));
+	VRM_CUDA(s, cudaStreamSynchronize(st));
+	trace.mark(st, "shadow horizon map");
 	if (buildMs) VRM_CUDA(s, cudaEventElapsedTime(buildMs, s->ev0, s->ev1));
 	return VRM_OK;
 }

@@ -196,6 +196,99 @@ struct LightWalk
 	uint32_t laPerm;  // pack_perm() of the ranked order
 };
 
+// ---- shadow horizon map --------------------------------------------------------------------------------------------------
+// A shadow ray's whole result is one bit (colour * !inShadow) and it travels along the light direction n.  The map is a 2D grid on
+// the plane perpendicular to n; a cell holds an upper bound of dot(X, n) over every point X of every occupied 8^3 cluster whose
+// projection, widened by kHorizonR, covers the cell.  A shadow ray looks its start point up once (every later point of its line
+// projects to the same place) and, once its depth along n is past the cell's value plus kHorizonMargin, no voxel test it can still
+// make can find an occupied cluster: it finishes lit, exactly as the full walk out of the scene would.
+// Coordinates are relative to the region table's origin (64 * minCoord), so scenes near +-2^23 lose nothing.
+//
+// kHorizonR bounds how far off the ray's exact line a tested voxel can lie, kHorizonMargin how far AHEAD along n (both in voxels):
+//   - any point of a tested voxel cube [g, g + 1]^3 lies within sqrt(3) of the ray point g was taken from (truncation);
+//   - the longest-axis walk tests g + axisDiff, taken from its origin `ro`, which runs up to one scaled step (|sd| <= sqrt(3)) ahead
+//     of o; its prologue steps back by at most one voxel, and the first voxel test after entering a region takes the voxel under the
+//     rebased position (coordinate up to 64, aliased into the same cluster grid);
+//   - fp32 drift of the walk in region-local coordinates: each advance rounds every coordinate by <= 2^-18 (|o| <= 64) and a ray
+//     makes far fewer than 10^4 advances outside crawls; a crawl (t = 0 on a face) cannot slide along a face for more than one
+//     iteration per axis when every non-zero |n_i| >= kHorizonMinComponent (kEps * |n_i| moves the coordinate off the face), which
+//     horizon_setup requires -- other lights get no map;
+//   - projection and lookup in fp32 (coordinates < 2^18): < 0.05; the splat adds one more voxel of padding for it.
+// sqrt(3) + sqrt(3) + 1 + drift < 4.5: R = 5 and margin = 5 voxels.  (The cell is 8+ voxels wide, so a larger R costs little.)
+constexpr float kHorizonR = 5.0f;
+constexpr float kHorizonMargin = 5.0f;
+constexpr float kHorizonClusterR = 6.92820323f;    // 4 * sqrt(3): circumradius of an 8^3 cluster around its centre
+constexpr double kHorizonMinComponent = 0.0625;    // lights with 0 < |n_i| < this get no map (see above)
+constexpr uint32_t kHorizonMaxCells = 2048;        // per side: the cell grows past 8 voxels for scenes wider than that
+constexpr int32_t kHorizonEmpty = (int32_t)0x80808080u;  // a cell no cluster covers (below every real value; a byte memset fills it)
+
+struct HorizonView
+{
+	const int32_t* cells;  // [nv][nu] ceil(max dot(X, n)) over the covering clusters, kHorizonEmpty if none; null: no map (rays walk out)
+	float n[3];            // unit light direction, world axes
+	float e1[3], e2[3];    // orthonormal basis of the plane perpendicular to n
+	float u0, v0, invCell; // cell (iu, iv) = floor((dot(X, e1) - u0) * invCell), floor((dot(X, e2) - v0) * invCell)
+	uint32_t nu, nv;
+	int axis;              // world axis of the largest |n_i|: the coordinate a shadow ray's threshold is stated in
+};
+
+// Grid for a scene of diameter D regions and light direction dir (host, double).  Returns false when the light gets no map.
+inline bool horizon_setup(const float* dir, uint32_t D, uint32_t permAxis0, HorizonView& h)
+{
+	h.cells = nullptr;
+	const double l = sqrt((double)dir[0] * dir[0] + (double)dir[1] * dir[1] + (double)dir[2] * dir[2]);
+	if (!(l > 0.0) || D == 0u) return false;
+	double n[3];
+	for (int i = 0; i < 3; i++)
+	{
+		n[i] = dir[i] / l;
+		if (n[i] != 0.0 && fabs(n[i]) < kHorizonMinComponent) return false;
+	}
+	const int k = fabs(n[0]) <= fabs(n[1]) ? (fabs(n[0]) <= fabs(n[2]) ? 0 : 2) : (fabs(n[1]) <= fabs(n[2]) ? 1 : 2);  // least aligned axis
+	double a[3] = {0.0, 0.0, 0.0};
+	a[k] = 1.0;
+	double e1[3] = {n[1] * a[2] - n[2] * a[1], n[2] * a[0] - n[0] * a[2], n[0] * a[1] - n[1] * a[0]};
+	const double l1 = sqrt(e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2]);
+	for (int i = 0; i < 3; i++) e1[i] /= l1;
+	const double e2[3] = {n[1] * e1[2] - n[2] * e1[1], n[2] * e1[0] - n[0] * e1[2], n[0] * e1[1] - n[1] * e1[0]};
+	const double side = 64.0 * D, pad = kHorizonClusterR + kHorizonR + 2.0;
+	double umin = 1e300, umax = -1e300, vmin = 1e300, vmax = -1e300;
+	for (int c = 0; c < 8; c++)
+	{
+		const double p[3] = {(c & 1) ? side : 0.0, (c & 2) ? side : 0.0, (c & 4) ? side : 0.0};
+		const double u = p[0] * e1[0] + p[1] * e1[1] + p[2] * e1[2], v = p[0] * e2[0] + p[1] * e2[1] + p[2] * e2[2];
+		umin = fmin(umin, u); umax = fmax(umax, u); vmin = fmin(vmin, v); vmax = fmax(vmax, v);
+	}
+	umin -= pad; vmin -= pad; umax += pad; vmax += pad;
+	double cell = 8.0;
+	while ((umax - umin) / cell >= kHorizonMaxCells || (vmax - vmin) / cell >= kHorizonMaxCells) cell *= 2.0;
+	for (int i = 0; i < 3; i++) { h.n[i] = (float)n[i]; h.e1[i] = (float)e1[i]; h.e2[i] = (float)e2[i]; }
+	h.u0 = (float)umin; h.v0 = (float)vmin; h.invCell = (float)(1.0 / cell);  // (a power of two)
+	h.nu = (uint32_t)((umax - umin) / cell) + 1u;
+	h.nv = (uint32_t)((vmax - vmin) / cell) + 1u;
+	h.axis = (int)permAxis0;  // rank_axes' longest axis of the light (ties broken as the shadow rays' walk space breaks them)
+	return true;
+}
+
+// One occupied cluster (cx, cy, cz: cluster coordinates relative to the table origin, 8 voxels each) -> max into every cell its
+// widened projection touches.  `update(cellIndex, value)` is atomicMax on the device, a plain max on the host.
+template <class F>
+VRM_HD void horizon_splat(const HorizonView& h, uint32_t cx, uint32_t cy, uint32_t cz, F update)
+{
+	const double p[3] = {8.0 * cx + 4.0, 8.0 * cy + 4.0, 8.0 * cz + 4.0};
+	const double u = p[0] * h.e1[0] + p[1] * h.e1[1] + p[2] * h.e1[2] - h.u0;
+	const double v = p[0] * h.e2[0] + p[1] * h.e2[1] + p[2] * h.e2[2] - h.v0;
+	const double depth = p[0] * h.n[0] + p[1] * h.n[1] + p[2] * h.n[2];
+	const double rr = (double)kHorizonClusterR + (double)kHorizonR + 1.0;  // + 1: fp32 projection at lookup
+	const int32_t val = (int32_t)ceil(depth + (double)kHorizonClusterR + 1.0);
+	const double ic = h.invCell;
+	int iu0 = (int)floor((u - rr) * ic), iu1 = (int)floor((u + rr) * ic), iv0 = (int)floor((v - rr) * ic), iv1 = (int)floor((v + rr) * ic);
+	iu0 = iu0 < 0 ? 0 : iu0; iv0 = iv0 < 0 ? 0 : iv0;
+	iu1 = iu1 >= (int)h.nu ? (int)h.nu - 1 : iu1; iv1 = iv1 >= (int)h.nv ? (int)h.nv - 1 : iv1;
+	for (int iv = iv0; iv <= iv1; iv++)
+		for (int iu = iu0; iu <= iu1; iu++) update((uint32_t)iv * h.nu + (uint32_t)iu, val);
+}
+
 struct HashRegionDesc  // 16 bytes, one LDG.128 per region entry
 {
 	uint32_t slotBase;  // first 64-bit slot of table 1; table 2 follows at slotBase + n
@@ -429,6 +522,9 @@ template <int ST, bool STATS> struct RayCtx
 	// 1: a hit whose shaded colour is already black starts no shadow ray (Renderer.cuh:314-315: 0 * !isInShadow = 0 whatever the shadow
 	// ray finds).  0 (host harness, reference-comparable event counters): every hit's shadow ray is traced, as the reference does.
 	uint32_t skipDead;
+	// Shadow horizon map (null cells: none).  Set only by the kernels that run the state machine of vrm_flat.cuh, and never for
+	// reference-comparable event counters (it ends lit shadow rays before the reference's walk does).
+	HorizonView hv;
 #if VRM_SMEM_MASK
 	// A/B form (north-star "shared-memory staging of cluster headers", DESIGN.md 3.2): the warp's copy of ONE region's 512-bit
 	// cluster-exists mask in shared memory and the region it belongs to (warp-uniform; -1 = none).  Filled by march_scene_flat_warp.
@@ -445,6 +541,7 @@ template <int ST, bool STATS> struct RayCtx
 		hit[0] = hit[1] = hit[2] = hit[3] = 0;
 		deferQueue = nullptr;
 		skipDead = 0u;
+		hv.cells = nullptr;
 		if (STATS) { st.nExist = st.nExistFalse = st.nLookup = st.nLookupHit = st.nProbe2 = st.nRegionReads = st.nCrawlSkipped = 0; }
 	}
 };

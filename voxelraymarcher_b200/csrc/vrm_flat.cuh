@@ -74,6 +74,8 @@ constexpr uint32_t kFlShadowLA = 2u;     // ... walked with the longest-axis rou
 constexpr uint32_t kFlEq0 = 4u;          // t_i == tMin of the last kAdvNext / kAdvJump advance, walk slot i = bit 2 + i  (getNormalFromTValues)
 constexpr uint32_t kFlEqMask = 28u;
 constexpr int kFlPermShift = 8;
+constexpr int kFlHzShift = 14;           // bits 14-31: the shadow ray's horizon threshold, a signed integer (past_horizon); kHzNever: none
+constexpr int32_t kHzNever = 131071, kHzMin = -131072;
 constexpr int32_t kRiPending = -3;       // FlatRay::ri: the ray has left its region, rebase + table read still to do          // bits 8-13: world axis of walk slot 0 / 1 / 2, two bits each
 
 // What a ray does when it meets the region-face ping-pong pathology (FlatRay::pingpong_skip):
@@ -106,6 +108,9 @@ constexpr int kPpOff = 0, kPpDefer = 1, kPpInline = 2;
 #endif
 #ifndef VRM_FAST_LOOPS
 #define VRM_FAST_LOOPS 1   // the warp stays inside a fast block while every marching lane still qualifies
+#endif
+#ifndef VRM_HORIZON_AT
+#define VRM_HORIZON_AT 1   // where a shadow ray tests its horizon threshold: 0 after every cluster skip / jump / null-region skip, 1 when it changes region
 #endif
 #ifndef VRM_FAST_PATHS
 #define VRM_FAST_PATHS 1   // march_scene_flat_warp (VCS + longest axis): warp-uniform fast paths for all-jump / all-null-region passes (FlatRay::fast_jump)
@@ -249,6 +254,7 @@ struct FlatRay
 			o[i] = vsub(o[i], (float)(diff * kRegion));  // convertRayToLocalSpace(.., scale 1), Ray.cuh:14-17: the product with 1.0f is the identity
 		}
 		st = kStRegion;
+		if (VRM_HORIZON_AT == 1 && past_horizon()) { finish(result); return; }
 		if (!position_sane(o)) { ri = -2; return; }  // see position_sane (vrm_core.cuh)
 		read_region_entry(c);
 	}
@@ -256,7 +262,7 @@ struct FlatRay
 	// rayMarchVoxelScene / rayMarchVoxelSceneLongestAxis up to the first region (Renderer.cuh:338-378, 917-954)
 	VRM_HD void start_primary(RayCtx<ST, STATS>& c, const float* originW, const float* dirW, float scale)
 	{
-		fl = 0; result = 0; ri = -2; seq = 0; ad1 = ad2 = 0;
+		fl = (uint32_t)kHzNever << kFlHzShift; result = 0; ri = -2; seq = 0; ad1 = ad2 = 0;
 		g[0] = g[1] = g[2] = 0; ro[0] = ro[1] = ro[2] = 0.0f;
 		PermRuntime p;
 		p.a0 = 0; p.a1 = 1; p.a2 = 2;
@@ -366,8 +372,41 @@ struct FlatRay
 			for (int i = 0; i < 3; i++) { d[i] = c.lw.idD[i]; rd[i] = c.lw.idR[i]; }
 			thr = c.lw.idThr;
 		}
+		fl |= (uint32_t)(c.hv.cells ? horizon_threshold(c, ss) : kHzNever) << kFlHzShift;
 		st = kStRegion;
 		read_region_entry(c);
+	}
+
+	// The shadow ray's threshold from ONE lookup of the horizon map at its start point (every later point of its line projects to the
+	// same place).  Stated in the signed world coordinate of the ray's walk slot 0 -- a = hv.axis (the largest |n_a|) for the longest-axis
+	// routine, world x for the original one (none when n_x = 0): the depth along n grows by 1 / |n_a| per unit of that coordinate.
+	// Rounded up to whole voxels and clamped to 18 bits, it travels in the flag word instead of a register of its own: coordinates
+	// relative to the table origin stay below 64 * 1024 = 65536, so kHzNever is never passed and kHzMin ends the ray at once.
+	VRM_HD int32_t horizon_threshold(const RayCtx<ST, STATS>& c, const ShadowStart& ss) const
+	{
+		const HorizonView& h = c.hv;
+		const int minC = c.sv.minCoord;
+		float pw[3];
+		for (int i = 0; i < 3; i++) pw[i] = (float)((ss.regW[i] - minC) * kRegion) + ss.hitW[i];  // relative to the table origin
+		int iu = (int)floorf((pw[0] * h.e1[0] + pw[1] * h.e1[1] + pw[2] * h.e1[2] - h.u0) * h.invCell);
+		int iv = (int)floorf((pw[0] * h.e2[0] + pw[1] * h.e2[1] + pw[2] * h.e2[2] - h.v0) * h.invCell);
+		iu = iu < 0 ? 0 : (iu >= (int)h.nu ? (int)h.nu - 1 : iu);  // (a start point off the grid has no cluster near its line at all)
+		iv = iv < 0 ? 0 : (iv >= (int)h.nv ? (int)h.nv - 1 : iv);
+		const int32_t top = ldg(h.cells + ((uint32_t)iv * h.nu + (uint32_t)iu));
+		const float depth0 = pw[0] * h.n[0] + pw[1] * h.n[1] + pw[2] * h.n[2];
+		const int a = (fl & kFlShadowLA) ? h.axis : 0;
+		const float na = pick3(a, h.n[0], h.n[1], h.n[2]), pa = pick3(a, pw[0], pw[1], pw[2]);
+		if (na == 0.0f) return kHzNever;
+		const float t = ceilf((na < 0.0f ? -pa : pa) + ((float)top + kHorizonMargin - depth0) * fabsf(na));
+		return t >= (float)kHzNever ? kHzNever : (t <= (float)kHzMin ? kHzMin : (int32_t)t);
+	}
+
+	// a shadow ray beyond its threshold: every voxel test it could still make lies past the deepest occupied cluster near its line
+	VRM_HD bool past_horizon() const
+	{
+		if (!(fl & kFlShadow)) return false;  // (primary rays hold kHzNever; the test only saves them the arithmetic)
+		const float w = (float)(ur[0] * (uint32_t)kRegion) + o[0];
+		return (d[0] < 0.0f ? -w : w) > (float)((int32_t)fl >> kFlHzShift);
 	}
 
 	VRM_HD void do_hit(RayCtx<ST, STATS>& c)
@@ -544,6 +583,7 @@ struct FlatRay
 		const float a0 = div_by_const(x0, sd[0], srd[0]), a1 = div_by_const(x1, sd[1], srd[1]), a2 = div_by_const(x2, sd[2], srd[2]);
 		const float s = vadd(min3(a0, a1, a2), kEps);  // the jump guards nothing (Renderer.cuh:457-459) and its tMin includes +EPSILON (713-716)
 		o[0] = along(o[0], s, sd[0]); o[1] = along(o[1], s, sd[1]); o[2] = along(o[2], s, sd[2]);
+		if (VRM_HORIZON_AT == 0 && past_horizon()) { finish(result); return true; }
 		// The equality bits of this advance (which t equals tMin, for the normal) are only ever read by a hit of the voxel test that
 		// follows in this very step: the next advance that can precede a hit -- another jump or the original algorithm's kAdvNext --
 		// rewrites them, a kAdvCluster only ever follows a kAdvNext, and longest-axis test hits take their normal from the slot.  So
@@ -591,6 +631,7 @@ struct FlatRay
 		const float a0 = div_by_const(x0, d[0], rd[0]), a1 = div_by_const(x1, d[1], rd[1]), a2 = div_by_const(x2, d[2], rd[2]);
 		const float s = min3(a0, a1, a2);
 		o[0] = along(o[0], s, d[0]); o[1] = along(o[1], s, d[1]); o[2] = along(o[2], s, d[2]);
+		if (VRM_HORIZON_AT == 0 && past_horizon()) { finish(result); return true; }
 		change_region(c);
 		enter_stored_region(c);
 		return true;
@@ -665,6 +706,8 @@ struct FlatRay
 				fl = (fl & ~kFlEqMask) | (a0 == tm ? kFlEq0 : 0u) | (a1 == tm ? kFlEq0 << 1 : 0u) | (a2 == tm ? kFlEq0 << 2 : 0u);
 			}
 			o[0] = along(o[0], s, e0); o[1] = along(o[1], s, e1); o[2] = along(o[2], s, e2);
+			// the tails of lit shadow rays are cluster skips / jumps and null-region skips through empty air (primary rays: kHzNever)
+			if (VRM_HORIZON_AT == 0 && mode >= kAdvCluster && past_horizon()) { finish(result); return; }
 			// grid_in_region((int)floorf(o)) of the jump (Renderer.cuh:719-723) and isRayInRegion(o) agree for every o
 			if (skip || !ray_in_region(o)) { change_region(c); return; }
 			g[0] = (int)o[0]; g[1] = (int)o[1]; g[2] = (int)o[2];  // == (int)floorf(o) inside a region

@@ -48,6 +48,11 @@ struct vrm_scene
 	uint32_t* d_values = nullptr;
 
 	vrm::Lighting light;
+	// shadow horizon map of the built scene for `light` (vrm_core.cuh HorizonView; cells null: none): rebuilt by vrm_set_lighting when
+	// the direction or use_shadows changes; VRM_SHADOW_HORIZON=0 at vrm_scene_create turns it off (A/B)
+	vrm::HorizonView horizon = {};
+	int32_t* d_horizon = nullptr;     size_t horizonCap = 0;  // cells allocated
+	bool horizonEnabled = true;
 
 	// scratch owned by the handle for the host-buffer entry points
 	int32_t* d_hits = nullptr;   size_t hitsBytes = 0;
@@ -132,6 +137,7 @@ inline int vrm_check_staging(vrm_scene* s)
 // vrm_build.cu
 int vrm_build_structure(vrm_scene* s, int storageType, float* buildMs);
 void vrm_free_structure(vrm_scene* s);
+int vrm_build_horizon(vrm_scene* s);  // (re)build s->horizon for s->light on s->stream, or drop it when the light gets none
 // Staging (vrm_build.cu).  vrm_stage_reserve: flush the host block, make room for `extra` more voxels and return where they go;
 // the caller fills them on s->stream (copy or kernel) and then calls vrm_stage_commit, which folds them into the running region
 // extent.  Nothing here synchronises the stream.

@@ -84,6 +84,7 @@ struct RenderArgs
 	unsigned int* shadowCtl;  // {records queued, next record to claim}
 	uint32_t shadowCap;
 	uint32_t skipDead;     // 1: a hit whose shaded colour is already black queues no shadow ray (0 * !shadow = 0)
+	HorizonView hv;        // shadow horizon map (cells null: none); read by the fused kernel (FORM 2) only
 };
 
 // ---- shadow-ray queue ------------------------------------------------------------------------------------------------------------
@@ -285,6 +286,7 @@ __global__ void __launch_bounds__(kRenderThreads, (FORM == 2 && VRM_FUSED_CTAS >
 		if constexpr (FORM == 2)
 		{
 			c.skipDead = a.skipDead;
+			c.hv = a.hv;
 #if VRM_SMEM_MASK
 			__shared__ uint32_t stagedMask[kRenderThreads / 32][16];
 			c.smMask = stagedMask[warp];
@@ -689,6 +691,7 @@ struct TraceArgs
 	unsigned int* shadowCtl;
 	uint32_t shadowCap;
 	uint32_t skipDead;
+	HorizonView hv;        // shadow horizon map (cells null: none); read by trace_fused_kernel only
 	const uint32_t* order; // null: thread t of the launch traces ray first + t; else ray first + order[t] (rays ordered for coherence, below)
 };
 
@@ -815,6 +818,7 @@ __global__ void __launch_bounds__(kTraceFusedThreads, VRM_FUSED_CTAS > 0 ? VRM_F
 	c.reset();
 	c.deferQueue = a.defer;
 	c.skipDead = a.skipDead;
+	c.hv = a.hv;
 	float o[3] = {0.0f, 0.0f, 0.0f}, d[3] = {0.0f, 0.0f, 0.0f};
 	if (live)
 	{
@@ -1045,6 +1049,9 @@ template <class Args> void fill_common(Args& a, const vrm_scene* s, const float*
 	a.defer = nullptr;
 	a.parkBits = nullptr; a.parkCtl = nullptr;
 	a.shadowItems = nullptr; a.shadowCtl = nullptr; a.shadowCap = 0; a.skipDead = 0;
+	// the horizon map ends lit shadow rays before the reference's walk does: never with reference-comparable event counters
+	a.hv = s->horizon;
+	if (s->statsMode == 1) a.hv.cells = nullptr;
 }
 
 // Shadow-ray queue of the handle: room for `records` records (grow-only), counters zeroed on the stream.
