@@ -281,6 +281,38 @@ int vrm_scene_read_voxels(vrm_scene* scene, const int32_t origin[3], const uint3
 int vrm_scene_read_voxels_device(vrm_scene* scene, const int32_t origin[3], const uint32_t dims[3], int32_t* d_xyz_out, uint32_t* d_rgb_out,
                                  uint64_t capacity, uint64_t* n_out);
 
+/* ---- hit surfaces --------------------------------------------------------------------------------------------------------
+ * How far away each hit is and which face the ray entered through, computed from a hit map the render / trace calls wrote (hits_out:
+ * global voxel x, y, z and a 0/1 flag per pixel or ray) and the exact ray.  The reference has no such output (it writes RGB8 only).
+ * DEFINITION (IEEE fp32, round to nearest, no contraction; one function, vrm_core.cuh hit_surface, serves the kernel and the tests):
+ *   ray:   views -- the pixel's ray of the render: image-plane origin P, unit direction D and len = |P - camera origin| (calculateWorldRay);
+ *          rays  -- P = rays[6i .. 6i+2], D = rays[6i+3 .. 6i+5].
+ *   local origin s_a = (float)scale * (P_a - translation_a), the transform the traversal applies.
+ *   For every axis a (x, y, z in that order) with D_a != 0: t_a = ((float)(D_a > 0 ? h_a : h_a + 1) - s_a) / D_a.  t = the largest t_a,
+ *   ties to the earlier axis; that axis gives face = 1 + 2a + (D_a < 0).
+ *   depth = len + t / (float)scale for views (world distance from the camera origin along the pixel's ray), t / (float)scale for rays
+ *   (world ray parameter: P + depth * D is the entry point).
+ *   flag 0: depth +inf, face 0.  No axis with D_a != 0 (never a camera ray): depth NaN, face 0.
+ *   Not clamped: a ray depth below 0 (a view depth below len) means the origin lies inside the hit voxel, or the traversal's accumulated
+ *   rounding reported a voxel the exact ray only grazes.
+ * Layouts: views take the hit map as vrm_render[_views]_device writes it, n_views x height x width x 4 int32 (view-major, row 0 = top);
+ * depth_out = n_views x height x width float32 and face_out = the same count of uint8 (rays: n each).  depth_out and face_out are each
+ * nullable, not both (VRM_ERR_INVALID).  Zero records return VRM_OK and write nothing.  The calls depend only on their arguments -- the
+ * handle lends its device, stream and scratch buffers -- and are legal before and after vrm_scene_build.
+ *   host variants: synchronous; hits, rays and outputs travel through the handle's device buffers.
+ *   device variants: asynchronous on the handle's stream; d_hits must be 16-byte aligned, d_depth_out and d_rays 4-byte aligned
+ *                    (VRM_ERR_INVALID otherwise); cameras stay a HOST array of n_views x 15 floats.
+ * Cost: one streaming pass, 16 bytes read and 5 written per record (DESIGN.md §3.6). */
+/* face codes: 0 = no hit, 1..6 = -x, +x, -y, +y, -z, +z (outward normal of the entered face) */
+int vrm_hit_surface_views(vrm_scene* scene, const float* cameras, uint32_t n_views, const float translation[3], uint32_t scale,
+                          uint32_t width, uint32_t height, const int32_t* hits, float* depth_out, uint8_t* face_out);
+int vrm_hit_surface_views_device(vrm_scene* scene, const float* cameras, uint32_t n_views, const float translation[3], uint32_t scale,
+                                 uint32_t width, uint32_t height, const int32_t* d_hits, float* d_depth_out, uint8_t* d_face_out);
+int vrm_hit_surface_rays(vrm_scene* scene, const float* rays, uint64_t n, const float translation[3], uint32_t scale,
+                         const int32_t* hits, float* depth_out, uint8_t* face_out);
+int vrm_hit_surface_rays_device(vrm_scene* scene, const float* d_rays, uint64_t n, const float translation[3], uint32_t scale,
+                                const int32_t* d_hits, float* d_depth_out, uint8_t* d_face_out);
+
 /* Opt-in L2 residency hint: an access-policy window (persisting) over the structure's hottest array -- the VCS cluster
  * headers or the hash table's slots -- on the handle's current stream (also VRM_L2_PERSIST=1 at vrm_scene_create).  Off by
  * default: on the BASELINE scenes the touched working set already lives in L1/L2 and the window measured no gain. */

@@ -38,7 +38,11 @@ EXPORTS = [
     "vrm_scene_set_completion_flag", "vrm_scene_set_completion_counter", "vrm_claim_next", "vrm_wait_flags_device", "vrm_render_views_sharded",
     "vrm_scene_add_dense", "vrm_scene_add_dense_device", "vrm_scene_read_box", "vrm_scene_read_box_device",
     "vrm_scene_read_voxels", "vrm_scene_read_voxels_device",
+    "vrm_hit_surface_views", "vrm_hit_surface_views_device", "vrm_hit_surface_rays", "vrm_hit_surface_rays_device",
 ]
+
+# face codes of the hit surfaces -> outward normal of the face the ray entered through (0 = no hit, then -x, +x, -y, +y, -z, +z)
+FACE_NORMALS = np.array([[0, 0, 0], [-1, 0, 0], [1, 0, 0], [0, -1, 0], [0, 1, 0], [0, 0, -1], [0, 0, 1]], np.int8)
 
 
 class VrmError(RuntimeError):
@@ -109,6 +113,10 @@ def load_library():
         "vrm_scene_read_box_device": (ci, [vp, vp, vp, vp]),
         "vrm_scene_read_voxels": (ci, [vp, vp, vp, vp, vp, u64, C.POINTER(u64)]),
         "vrm_scene_read_voxels_device": (ci, [vp, vp, vp, vp, vp, u64, C.POINTER(u64)]),
+        "vrm_hit_surface_views": (ci, [vp, vp, u32, vp, u32, u32, u32, vp, vp, vp]),
+        "vrm_hit_surface_views_device": (ci, [vp, vp, u32, vp, u32, u32, u32, vp, vp, vp]),
+        "vrm_hit_surface_rays": (ci, [vp, vp, u64, vp, u32, vp, vp, vp]),
+        "vrm_hit_surface_rays_device": (ci, [vp, vp, u64, vp, u32, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -377,15 +385,20 @@ class VoxelScene:
         return np.ascontiguousarray(camera.data if isinstance(camera, Camera) else camera, np.float32)
 
     def run_raymarching_kernel(self, width, height, algorithm, camera, scale=1, translation=(0.0, 0.0, 0.0), want_hits=False,
-                               rgb_out=None):
-        """Render one frame into host memory.  Returns dict(rgb[H,W,3] uint8, hits[H,W,4] int32 | None, kernel_ms)."""
+                               rgb_out=None, want_surface=False):
+        """Render one frame into host memory.  Returns dict(rgb[H,W,3] uint8, hits[H,W,4] int32 | None, kernel_ms); with
+        ``want_surface`` also depth[H,W] float32 and face[H,W] uint8 of ``hit_surface_views`` (the hit map is then rendered internally)."""
         rgb = rgb_out if rgb_out is not None else np.zeros((height, width, 3), np.uint8)
-        hits = np.zeros((height, width, 4), np.int32) if want_hits else None
+        hits = np.zeros((height, width, 4), np.int32) if want_hits or want_surface else None
         ms = C.c_float()
         cam = self._cam(camera)
         self._check(self.lib.vrm_render(self.h, _ptr(cam), _ptr(_f3(translation)), scale, self._algo(algorithm), width, height,
                                         _ptr(rgb), _ptr(hits), C.byref(ms)), "vrm_render")
-        return dict(rgb=rgb, hits=hits, kernel_ms=ms.value)
+        out = dict(rgb=rgb, hits=hits if want_hits else None, kernel_ms=ms.value)
+        if want_surface:
+            depth, face = self.hit_surface_views(hits, [cam], width, height, scale, translation)
+            out.update(depth=depth[0], face=face[0])
+        return out
 
     render = run_raymarching_kernel
 
@@ -416,20 +429,71 @@ class VoxelScene:
                                               _ptr(rgb_out), C.byref(ms)), "vrm_render_views")
         return {"rgb": rgb_out.reshape(n, height, width, 3), "total_ms": ms.value}
 
-    def trace_rays(self, rays, algorithm, scale=1, translation=(0.0, 0.0, 0.0), want_hits=False):
+    def trace_rays(self, rays, algorithm, scale=1, translation=(0.0, 0.0, 0.0), want_hits=False, want_surface=False):
+        """Trace world rays (n, 6).  Returns dict(colour (n,) uint32, hits (n, 4) int32 | None, kernel_ms); with ``want_surface`` also
+        depth (n,) float32 and face (n,) uint8 of ``hit_surface_rays`` (the hit records are then traced internally)."""
         rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 6)
         n = rays.shape[0]
         colour = np.zeros(n, np.uint32)
-        hits = np.zeros((n, 4), np.int32) if want_hits else None
+        hits = np.zeros((n, 4), np.int32) if want_hits or want_surface else None
         ms = C.c_float()
         self._check(self.lib.vrm_trace_rays(self.h, _ptr(rays), n, _ptr(_f3(translation)), scale, self._algo(algorithm), _ptr(colour),
                                             _ptr(hits), C.byref(ms)), "vrm_trace_rays")
-        return dict(colour=colour, hits=hits, kernel_ms=ms.value)
+        out = dict(colour=colour, hits=hits if want_hits else None, kernel_ms=ms.value)
+        if want_surface:
+            out["depth"], out["face"] = self.hit_surface_rays(hits, rays, scale, translation)
+        return out
 
     def trace_rays_device(self, d_rays_ptr: int, n: int, algorithm, d_colour_ptr: int, d_hits_ptr: int | None = None, scale=1,
                           translation=(0.0, 0.0, 0.0)):
         self._check(self.lib.vrm_trace_rays_device(self.h, C.c_void_p(d_rays_ptr), n, _ptr(_f3(translation)), scale, self._algo(algorithm),
                                                    C.c_void_p(d_colour_ptr), C.c_void_p(d_hits_ptr or 0)), "vrm_trace_rays_device")
+
+    # -- hit surfaces (include/vrm_b200.h "hit surfaces": depth and entered face from a hit map and the exact ray) -----------------
+    def hit_surface_views(self, hits, cameras, width, height, scale=1, translation=(0.0, 0.0, 0.0)):
+        """Depth and face of a view-major hit map ``hits`` (n, H, W, 4) int32 as ``render`` / ``render_views_device`` write it, for the
+        n ``cameras`` it was rendered with.  Returns (depth (n, H, W) float32, face (n, H, W) uint8): depth = world distance from the
+        camera origin along the pixel's ray (+inf for a miss), face = 1..6 for -x, +x, -y, +y, -z, +z (``FACE_NORMALS``), 0 for a miss."""
+        cams = np.ascontiguousarray(np.stack([self._cam(c) for c in cameras]), np.float32)
+        n = cams.shape[0]
+        hits = np.ascontiguousarray(hits, np.int32)
+        if hits.size != n * height * width * 4:
+            raise ValueError(f"hits holds {hits.size // 4} records, {n} views of {width}x{height} need {n * height * width}")
+        depth = np.empty((n, height, width), np.float32)
+        face = np.empty((n, height, width), np.uint8)
+        self._check(self.lib.vrm_hit_surface_views(self.h, _ptr(cams), n, _ptr(_f3(translation)), int(scale), width, height, _ptr(hits),
+                                                   _ptr(depth), _ptr(face)), "vrm_hit_surface_views")
+        return depth, face
+
+    def hit_surface_views_device(self, d_hits_ptr: int, cameras, width, height, d_depth_ptr: int | None, d_face_ptr: int | None, scale=1,
+                                 translation=(0.0, 0.0, 0.0)):
+        """``hit_surface_views`` on device buffers (e.g. ``tensor.data_ptr()``; hits 16-byte aligned, depth 4-byte aligned; either output
+        may be None); asynchronous on the scene's stream."""
+        cams = np.ascontiguousarray(np.stack([self._cam(c) for c in cameras]), np.float32)
+        self._check(self.lib.vrm_hit_surface_views_device(self.h, _ptr(cams), cams.shape[0], _ptr(_f3(translation)), int(scale), width, height,
+                                                          C.c_void_p(d_hits_ptr), C.c_void_p(d_depth_ptr or 0), C.c_void_p(d_face_ptr or 0)),
+                    "vrm_hit_surface_views_device")
+
+    def hit_surface_rays(self, hits, rays, scale=1, translation=(0.0, 0.0, 0.0)):
+        """Depth and face of traced rays (n, 6) and their hit records (n, 4) from ``trace_rays``.  Returns (depth (n,) float32, face (n,)
+        uint8): depth = world ray parameter of the entry point (origin + depth * direction), +inf for a miss."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 6)
+        n = rays.shape[0]
+        hits = np.ascontiguousarray(hits, np.int32)
+        if hits.size != n * 4:
+            raise ValueError(f"hits holds {hits.size // 4} records for {n} rays")
+        depth = np.empty(n, np.float32)
+        face = np.empty(n, np.uint8)
+        self._check(self.lib.vrm_hit_surface_rays(self.h, _ptr(rays), n, _ptr(_f3(translation)), int(scale), _ptr(hits), _ptr(depth), _ptr(face)),
+                    "vrm_hit_surface_rays")
+        return depth, face
+
+    def hit_surface_rays_device(self, d_hits_ptr: int, d_rays_ptr: int, n: int, d_depth_ptr: int | None, d_face_ptr: int | None, scale=1,
+                                translation=(0.0, 0.0, 0.0)):
+        """``hit_surface_rays`` on device buffers (hits 16-byte aligned, rays and depth 4-byte aligned); asynchronous on the scene's stream."""
+        self._check(self.lib.vrm_hit_surface_rays_device(self.h, C.c_void_p(d_rays_ptr), int(n), _ptr(_f3(translation)), int(scale),
+                                                         C.c_void_p(d_hits_ptr), C.c_void_p(d_depth_ptr or 0), C.c_void_p(d_face_ptr or 0)),
+                    "vrm_hit_surface_rays_device")
 
     def lookup(self, xyz):
         xyz = np.ascontiguousarray(xyz, np.int32).reshape(-1, 3)

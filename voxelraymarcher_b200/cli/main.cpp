@@ -3,7 +3,8 @@
 // Same positional arguments, defaults (anything but the exact strings selects VCS / Longest Axis), prints, fixed
 // 1920x1080 frame and camera, `resources/scene.vox` input and `output.png` output as the reference.  Extras (all optional,
 // after the positional arguments): --scene PATH --out PATH --width W --height H --dump-voxels PATH (write the loaded voxel list as text and exit;
-// no device needed).
+// no device needed) --depth PATH (also write the frame's depth, vrm_hit_surface_views: world distance from the camera per pixel, +inf where
+// the ray hit nothing, as a little-endian grayscale PFM).
 //
 // Scene file: the reference's text format, one `x,y,z,color` line per voxel (geometry/VoxelFile.cuh:9-35); files that
 // start with the magic "VOX " are read as MagicaVoxel binaries instead (north star; the reference itself has no such
@@ -310,6 +311,22 @@ bool writePng(const std::string& path, const uint8_t* rgb, uint32_t w, uint32_t 
 	return bool(f);
 }
 
+// Grayscale PFM ("Pf", scale -1 = little-endian floats); PFM stores the bottom row first, the frame has row 0 at the top.
+bool writePfm(const std::string& path, const float* depth, uint32_t w, uint32_t h)
+{
+	std::ofstream f(path, std::ios::binary);
+	f << "Pf\n" << w << ' ' << h << "\n-1.0\n";
+	for (uint32_t y = h; y-- > 0;)
+		for (uint32_t x = 0; x < w; x++)
+		{
+			uint32_t bits;
+			memcpy(&bits, depth + size_t(y) * w + x, 4);
+			const char le[4] = {char(bits), char(bits >> 8), char(bits >> 16), char(bits >> 24)};
+			f.write(le, 4);
+		}
+	return bool(f);
+}
+
 }  // namespace
 
 int main(int argc, char* argv[])
@@ -325,7 +342,7 @@ int main(int argc, char* argv[])
 	else std::cout << "Storage Type: Voxel Cluster Storage" << std::endl;
 	if (argc > 3 && std::strcmp(argv[3], "original") == 0) { std::cout << "Raymarching Algorithm: Original" << std::endl; algorithm = VRM_ALGO_ORIGINAL; }  // Main.cu:58-68
 	else std::cout << "Raymarching Algorithm: Longest Axis" << std::endl;
-	std::string scenePath = "resources/scene.vox", outPath = "output.png";  // Main.cu:99,170; VoxelFile.cuh:12
+	std::string scenePath = "resources/scene.vox", outPath = "output.png", depthPath;  // Main.cu:99,170; VoxelFile.cuh:12
 	uint32_t width = 1920, height = 1080;                                   // Main.cu:195-196
 	for (int i = 4; i + 1 < argc; i += 2)
 	{
@@ -333,6 +350,7 @@ int main(int argc, char* argv[])
 		else if (!std::strcmp(argv[i], "--out")) outPath = argv[i + 1];
 		else if (!std::strcmp(argv[i], "--width")) width = uint32_t(std::stoul(argv[i + 1]));
 		else if (!std::strcmp(argv[i], "--height")) height = uint32_t(std::stoul(argv[i + 1]));
+		else if (!std::strcmp(argv[i], "--depth")) depthPath = argv[i + 1];
 	}
 
 	std::string dumpPath;
@@ -382,10 +400,18 @@ int main(int argc, char* argv[])
 	vrm_camera_make(origin, lookAt, up, 60.0f, aspect, cam);
 	float translation[3] = {0.0f, 0.0f, 0.0f}, kernelMs = 0.0f;  // Main.cu:215
 	std::vector<uint8_t> frame(size_t(width) * height * 3);
-	rc = vrm_render(scene, cam, translation, uint32_t(scale), algorithm, width, height, frame.data(), nullptr, &kernelMs);
+	std::vector<int32_t> hits(depthPath.empty() ? 0 : size_t(width) * height * 4);
+	rc = vrm_render(scene, cam, translation, uint32_t(scale), algorithm, width, height, frame.data(), depthPath.empty() ? nullptr : hits.data(), &kernelMs);
 	std::cout << (rc == VRM_OK ? "no error" : vrm_last_error(scene)) << std::endl;  // cudaGetErrorString(cudaPeekAtLastError()), Main.cu:154-155
 	std::cout << "Execution Time for Ray Marching Algorithm is: " << static_cast<long long>(kernelMs * 1000.0f) << " microseconds" << std::endl;  // Main.cu:162
 	if (rc == VRM_OK && !writePng(outPath, frame.data(), width, height)) std::cout << "ERROR: Failed to write image to: " << outPath << std::endl;  // ImageWriter.cpp:11-14
+	if (rc == VRM_OK && !depthPath.empty())
+	{
+		std::vector<float> depth(size_t(width) * height);
+		rc = vrm_hit_surface_views(scene, cam, 1, translation, uint32_t(scale), width, height, hits.data(), depth.data(), nullptr);
+		if (rc != VRM_OK) std::cout << "ERROR: " << vrm_error_string(rc) << ": " << vrm_last_error(scene) << std::endl;
+		else if (!writePfm(depthPath, depth.data(), width, height)) std::cout << "ERROR: Failed to write depth to: " << depthPath << std::endl;
+	}
 	vrm_scene_destroy(scene);
 	return rc == VRM_OK ? EXIT_SUCCESS : EXIT_FAILURE;
 }

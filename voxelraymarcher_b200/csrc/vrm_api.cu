@@ -61,10 +61,7 @@ void vrm_apply_l2_window(vrm_scene* s)
 	s->l2WindowStream = want ? s->stream : nullptr;
 }
 
-namespace
-{
-
-int ensure(vrm_scene* s, void** p, size_t* have, size_t need)
+int vrm_ensure(vrm_scene* s, void** p, size_t* have, size_t need)
 {
 	if (*have >= need && *p) return VRM_OK;
 	if (*p) { VRM_CUDA(s, cudaStreamSynchronize(s->stream)); cudaFree(*p); *p = nullptr; *have = 0; }
@@ -72,6 +69,9 @@ int ensure(vrm_scene* s, void** p, size_t* have, size_t need)
 	*have = need;
 	return VRM_OK;
 }
+
+namespace
+{
 
 int check_render_args(vrm_scene* s, const float* camera, const float* translation, int algorithm, uint32_t W, uint32_t H)
 {
@@ -82,7 +82,9 @@ int check_render_args(vrm_scene* s, const float* camera, const float* translatio
 	return VRM_OK;
 }
 
-int upload_cameras(vrm_scene* s, const float* cameras, uint32_t nViews)
+}  // namespace
+
+int vrm_upload_cameras(vrm_scene* s, const float* cameras, uint32_t nViews)
 {
 	size_t bytes = (size_t)nViews * VRM_CAMERA_FLOATS * sizeof(float);
 	if (s->camsBytes < bytes || !s->h_cams || !s->d_cams)
@@ -109,8 +111,6 @@ int upload_cameras(vrm_scene* s, const float* cameras, uint32_t nViews)
 	VRM_CUDA(s, cudaEventRecord(s->ev1, s->stream));
 	return VRM_OK;
 }
-
-}  // namespace
 
 extern "C" {
 
@@ -355,7 +355,7 @@ int vrm_render_views_device_strided(vrm_scene* s, const float* cameras, uint32_t
 	if (!d_rgb_out || n_views == 0 || n_views > 65535 || view_stride == 0) { s->lastError = "invalid render arguments"; return VRM_ERR_INVALID; }
 	VRM_CUDA(s, cudaSetDevice(s->device));
 	const bool inlineCam = n_views == 1 && vrm_camera_inline_ok(s);  // the camera of a single view travels in the kernel arguments
-	if (!inlineCam) { rc = upload_cameras(s, cameras, n_views); if (rc) return rc; }
+	if (!inlineCam) { rc = vrm_upload_cameras(s, cameras, n_views); if (rc) return rc; }
 	return vrm_launch_render(s, inlineCam ? nullptr : s->d_cams, n_views, translation, scale, algorithm, width, height, d_rgb_out, d_hits_out, 0, 0xFFFFFFFFu, view_stride,
 	                         inlineCam ? cameras : nullptr);
 }
@@ -410,7 +410,7 @@ int vrm_render(vrm_scene* s, const float camera[VRM_CAMERA_FLOATS], const float 
 		d_rgb = static_cast<uint8_t*>(device_alias(s->h_stage));
 		if (!d_rgb) { s->lastError = "page-locked staging frame is not mapped"; return VRM_ERR_CUDA; }
 	}
-	if (copyHits) { p = s->d_hits; rc = ensure(s, &p, &s->hitsBytes, px * 16); s->d_hits = static_cast<int32_t*>(p); if (rc) return rc; d_hits = s->d_hits; }
+	if (copyHits) { p = s->d_hits; rc = vrm_ensure(s, &p, &s->hitsBytes, px * 16); s->d_hits = static_cast<int32_t*>(p); if (rc) return rc; d_hits = s->d_hits; }
 	// Page-locked frame, copy-engine form (s->pinnedDma bands): the kernels render horizontal bands into a frame in device memory (per-warp
 	// stores, no PCIe traffic from the SMs) and the copy engine sends band k while band k+1 renders.  Full-line DMA writes instead of
 	// 96-byte partial-line stores from the SMs: what keeps the end-to-end rate up when eight GPUs write frames into host memory at once.
@@ -430,7 +430,7 @@ int vrm_render(vrm_scene* s, const float camera[VRM_CAMERA_FLOATS], const float 
 		d_rgb = s->d_dmaFrame;
 	}
 	const bool inlineCam = vrm_camera_inline_ok(s);  // the camera travels in the kernel arguments: nothing to upload
-	if (!inlineCam) { rc = upload_cameras(s, camera, 1); if (rc) return rc; }
+	if (!inlineCam) { rc = vrm_upload_cameras(s, camera, 1); if (rc) return rc; }
 	VRM_CUDA(s, cudaEventRecord(s->ev0, s->stream));
 	constexpr int kMaxBands = 8;
 	int bands = 1;
@@ -491,7 +491,7 @@ int vrm_render_views(vrm_scene* s, const float* cameras, uint32_t n_views, const
 		for (uint32_t v0 = 0; v0 < n_views; v0 += maxViewsPerLaunch)
 		{
 			const uint32_t nv = n_views - v0 < maxViewsPerLaunch ? n_views - v0 : maxViewsPerLaunch;
-			rc = upload_cameras(s, cameras + (size_t)v0 * VRM_CAMERA_FLOATS, nv);
+			rc = vrm_upload_cameras(s, cameras + (size_t)v0 * VRM_CAMERA_FLOATS, nv);
 			if (rc) return rc;
 			rc = vrm_launch_render(s, s->d_cams, nv, translation, scale, algorithm, width, height, mapped + (size_t)v0 * frameBytes, nullptr);
 			if (rc) return rc;
@@ -532,7 +532,7 @@ int vrm_render_views(vrm_scene* s, const float* cameras, uint32_t n_views, const
 			const int slot = (int)(batch & 1u);
 			const uint32_t nv = n_views - v0 < perBatch ? n_views - v0 : (uint32_t)perBatch;
 			if (batch >= 2) VRM_CUDA(s, cudaStreamWaitEvent(s->stream, s->evCopied[slot], 0));  // the buffer's previous batch has left the device
-			rc = upload_cameras(s, cameras + (size_t)v0 * VRM_CAMERA_FLOATS, nv);
+			rc = vrm_upload_cameras(s, cameras + (size_t)v0 * VRM_CAMERA_FLOATS, nv);
 			if (rc) return rc;
 			rc = vrm_launch_render(s, s->d_cams, nv, translation, scale, algorithm, width, height, s->d_batch[slot], nullptr);
 			if (rc) return rc;
@@ -573,7 +573,7 @@ int vrm_trace_rays(vrm_scene* s, const float* rays, uint64_t n, const float tran
 	if (n == 0) return VRM_OK;
 	VRM_CUDA(s, cudaSetDevice(s->device));
 	const size_t rayBytes = n * 24, colBytes = n * 4, hitBytes = hits_out ? n * 16 : 0;
-	int rc = ensure(s, &s->d_io, &s->ioBytes, rayBytes + colBytes + hitBytes);
+	int rc = vrm_ensure(s, &s->d_io, &s->ioBytes, rayBytes + colBytes + hitBytes);
 	if (rc) return rc;
 	char* base = static_cast<char*>(s->d_io);
 	int32_t* d_hits = hits_out ? reinterpret_cast<int32_t*>(base) : nullptr;  // 16-byte aligned first
@@ -598,7 +598,7 @@ int vrm_lookup(vrm_scene* s, const int32_t* xyz, uint64_t n, uint32_t* out, uint
 	if (n == 0) return VRM_OK;
 	VRM_CUDA(s, cudaSetDevice(s->device));
 	const size_t qBytes = n * 12, oBytes = n * 4, eBytes = n;
-	int rc = ensure(s, &s->d_io, &s->ioBytes, qBytes + oBytes + eBytes);
+	int rc = vrm_ensure(s, &s->d_io, &s->ioBytes, qBytes + oBytes + eBytes);
 	if (rc) return rc;
 	char* base = static_cast<char*>(s->d_io);
 	int32_t* d_q = reinterpret_cast<int32_t*>(base);

@@ -1341,8 +1341,9 @@ VRM_HD uint32_t march_scene(RayCtx<ST, STATS>& c, const float* originW, const fl
 	return ss.lit * (uint32_t)!shadow_nested<ST, ALGO, STATS>(c, ss);
 }
 
-// calculateWorldRay (Renderer.cuh:1013-1022) + Camera::generateRay (Camera.cuh:25-29).  cam = 15 floats.
-VRM_HD void primary_ray(const float* cam, uint32_t x, uint32_t y, uint32_t W, uint32_t H, float* o, float* d)
+// calculateWorldRay (Renderer.cuh:1013-1022) + Camera::generateRay (Camera.cuh:25-29).  cam = 15 floats.  len = |o - eye|, the
+// world distance from the camera origin to the ray's image-plane origin o.
+VRM_HD void primary_ray(const float* cam, uint32_t x, uint32_t y, uint32_t W, uint32_t H, float* o, float* d, float& len)
 {
 	float u = vdiv(vadd((float)x, 0.5f), (float)W);
 	float v = vdiv(vadd((float)(H - y), 0.5f), (float)H);
@@ -1352,8 +1353,44 @@ VRM_HD void primary_ray(const float* cam, uint32_t x, uint32_t y, uint32_t W, ui
 		o[i] = vadd(vadd(cam[3 + i], vmul(u, cam[6 + i])), vmul(v, cam[9 + i]));
 		rel[i] = vsub(o[i], cam[i]);
 	}
-	float len = vsqrt(vadd(vadd(vmul(rel[0], rel[0]), vmul(rel[1], rel[1])), vmul(rel[2], rel[2])));
+	len = vsqrt(vadd(vadd(vmul(rel[0], rel[0]), vmul(rel[1], rel[1])), vmul(rel[2], rel[2])));
 	d[0] = vdiv(rel[0], len); d[1] = vdiv(rel[1], len); d[2] = vdiv(rel[2], len);
+}
+
+VRM_HD void primary_ray(const float* cam, uint32_t x, uint32_t y, uint32_t W, uint32_t H, float* o, float* d)
+{
+	float len;
+	primary_ray(cam, x, y, W, H, o, d, len);
+}
+
+// ---------------------------------------------------------------- hit surfaces (vrm_hit_surface_*, DESIGN.md §3.6)
+//
+// Depth and entered face of a reported hit record hit = {x, y, z, flag} for the WORLD ray origin P, unit direction D: the exact ray
+// against the slabs of the hit voxel in local units, s = scale * (P - translation) as march_scene_primary transforms the origin.  For
+// every axis a with D_a != 0: t_a = (f_a - s_a) / D_a with f_a = D_a > 0 ? h_a : h_a + 1; t = the largest t_a, ties to the earlier
+// axis; face = 1 + 2a + (D_a < 0), so 1..6 = -x, +x, -y, +y, -z, +z, the outward normal of the face the ray enters through.
+//   depth = len + t / scale  (withLen: a camera ray, len from primary_ray -- the world distance from the eye along the pixel's ray)
+//         = t / scale        (a traced ray: the world ray parameter, P + depth * D is the entry point)
+// flag 0: +inf and face 0.  No axis with D_a != 0: NaN and face 0 (no camera ray).  Not clamped: a depth below len (below 0 for a
+// trace) means the origin lies inside the hit voxel, or the reference walk's drift reported a voxel the exact ray only grazes.
+// This one function is the definition: the sm_100a kernel (vrm_surface.cu) and the CPU tests' host build both call it.
+VRM_HD float hit_surface(const int32_t* hit, const float* P, const float* D, const float* translation, float scale, float len, bool withLen,
+                         uint32_t& face)
+{
+	face = 0u;
+	if (hit[3] == 0) return INFINITY;
+	float t = 0.0f;
+	for (int a = 0; a < 3; a++)
+	{
+		if (D[a] == 0.0f) continue;
+		const float s = vmul(scale, vsub(P[a], translation[a]));
+		const float f = (float)(D[a] > 0.0f ? hit[a] : hit[a] + 1);
+		const float ta = vdiv(vsub(f, s), D[a]);
+		if (face == 0u || ta > t) { t = ta; face = 1u + 2u * (uint32_t)a + (D[a] < 0.0f ? 1u : 0u); }
+	}
+	if (face == 0u) return NAN;
+	const float q = vdiv(t, scale);
+	return withLen ? vadd(len, q) : q;
 }
 
 }  // namespace vrm

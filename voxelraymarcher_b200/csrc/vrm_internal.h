@@ -160,6 +160,10 @@ void vrm_sort_pairs_u64(unsigned long long*& keys, uint32_t*& vals, unsigned lon
 
 // vrm_api.cu: install / remove the access-policy window on the handle's current stream (called by the launch wrappers)
 void vrm_apply_l2_window(vrm_scene* s);
+// vrm_api.cu: grow one of the handle's device buffers (*p, *have bytes) to at least `need` bytes (contents not kept), and stage
+// nViews cameras through the pinned buffer into s->d_cams on the handle's stream
+int vrm_ensure(vrm_scene* s, void** p, size_t* have, size_t need);
+int vrm_upload_cameras(vrm_scene* s, const float* cameras, uint32_t nViews);
 
 // vrm_multi.cu: publish the handle's next completion sequence number behind the launches already on its stream (no-op without a flag)
 void vrm_signal_completion(vrm_scene* s, uint32_t frames);
