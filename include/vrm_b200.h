@@ -313,6 +313,51 @@ int vrm_hit_surface_rays(vrm_scene* scene, const float* rays, uint64_t n, const 
 int vrm_hit_surface_rays_device(vrm_scene* scene, const float* d_rays, uint64_t n, const float translation[3], uint32_t scale,
                                 const int32_t* d_hits, float* d_depth_out, uint8_t* d_face_out);
 
+/* ---- exact ray casts -----------------------------------------------------------------------------------------------------
+ * The first STORED voxel (one vrm_scene_read_voxels lists) along the exact ray within a ray interval, with its entry depth, face and colour.
+ * Unlike vrm_trace_rays / vrm_render, which reproduce the reference's walks and their fp32 drift and always run to the first hit or out of
+ * the scene, the result is a pure function of the ray, and the walk ends at t_far.
+ * DEFINITION (IEEE fp32, round to nearest, no contraction; one function, vrm_core.cuh cast_ray, serves the kernel and the tests):
+ *   local frame: s_a = (float)scale * (P_a - translation_a) for the world origin P and direction D (any length); voxel c occupies
+ *     [c_a, c_a + 1) on each axis; the local parameter tau relates to the world ray parameter t by t = tau / scale, and the walk covers
+ *     tau0 = t_near * scale .. tau1 = t_far * scale.
+ *   plane crossings: for an axis with D_a != 0 (-0.0 counts as zero), plane k is crossed at tau_a(k) = ((float)k - s_a) / D_a -- the
+ *     expression of the hit surfaces; monotone in k, not strictly once |k - s_a| passes about 2^23.
+ *   start cell: the cell after every crossing with tau <= tau0: c_a = max{k : tau_a(k) <= tau0} for D_a > 0, min{k : tau_a(k + 1) <= tau0}
+ *     for D_a < 0, floorf(s_a) for D_a == 0 (a search on tau_a, not floor(s + tau0 * D), which rounds differently).
+ *   walk: repeatedly take the smallest next crossing, tau_a(c_a + 1) for D_a > 0 or tau_a(c_a) for D_a < 0, ties to the earlier axis
+ *     (x, y, z); stop when it is > tau1, else step c_a by +-1: the new cell was entered at that tau through face 1 + 2a + (D_a < 0).
+ *   result: the first cell of that sequence, the start cell included, holding a stored voxel; cells outside the region table's box
+ *     [64 * min_coord, 64 * (min_coord + diameter))^3 hold nothing.
+ *     hit in an entered cell: hits = {x, y, z, 1}, depth = tau / scale, face 1..6, colour = the stored colour, exactly what vrm_lookup
+ *       returns (VRM_EMPTY for a voxel stored with that colour);
+ *     hit in the start cell: depth = t_near exactly, face 0;
+ *     miss: hits {0, 0, 0, 0}, depth +inf, face 0, colour VRM_EMPTY.
+ *   always a miss: a non-finite origin, direction component or t_near, a NaN t_far, t_near > t_far, and a local origin or tau0 that is not
+ *     finite in fp32 (a non-finite translation, or an overflow).  A zero direction is legal: only the start cell is tested.
+ *   consequences: the depth of an entered-cell hit equals the hit surfaces' depth for that hit record (both take the largest entry-plane
+ *     tau), bit for bit except that an exact tie at tau = 0 may give +0 against -0; the face equals theirs except in exact ties between
+ *     axes, where the hit surfaces pick the earlier axis and the cast reports the axis it crossed last.  For a scale that is not a power of two, depth can round one ulp outside [t_near, t_far].
+ *   views: the pixel's ray of the render (image-plane origin P, unit D, len = |P - camera origin|) over [0, +inf); depth = len + tau / scale,
+ *     len for a start-cell hit -- the render's pixel ray traced exactly.  The hit map has the layout vrm_hit_surface_views reads.
+ * Layouts: rays = n x 6 floats (origin, direction); ranges = n x 2 floats {t_near, t_far}, NULL = [0, +inf) for every ray; views are
+ * view-major n_views x height x width, row 0 = top.  hits_out = records x 4 int32, depth_out float32, face_out uint8 (codes as above),
+ * colour_out uint32.  Each output is nullable, not all four (VRM_ERR_INVALID).  Legal only after vrm_scene_build (VRM_ERR_STATE before);
+ * scale 0 is VRM_ERR_INVALID; zero records return VRM_OK and write nothing.  Outputs are in the caller's ray order.
+ *   host variants: synchronous; rays, ranges and outputs travel through the handle's device buffers.
+ *   device variants: asynchronous on the handle's stream; d_hits_out must be 16-byte aligned, d_rays, d_ranges, d_depth_out and
+ *                    d_colour_out 4-byte aligned (VRM_ERR_INVALID otherwise); cameras stay a HOST array of n_views x 15 floats.
+ * Cost: the walk leaps over null 64^3 regions and empty 8^3 clusters exactly and steps cell by cell only inside occupied clusters
+ * (DESIGN.md §3.7). */
+int vrm_cast_rays(vrm_scene* scene, const float* rays, const float* ranges, uint64_t n, const float translation[3], uint32_t scale,
+                  int32_t* hits_out, float* depth_out, uint8_t* face_out, uint32_t* colour_out);
+int vrm_cast_rays_device(vrm_scene* scene, const float* d_rays, const float* d_ranges, uint64_t n, const float translation[3], uint32_t scale,
+                         int32_t* d_hits_out, float* d_depth_out, uint8_t* d_face_out, uint32_t* d_colour_out);
+int vrm_cast_views(vrm_scene* scene, const float* cameras, uint32_t n_views, const float translation[3], uint32_t scale, uint32_t width,
+                   uint32_t height, int32_t* hits_out, float* depth_out, uint8_t* face_out, uint32_t* colour_out);
+int vrm_cast_views_device(vrm_scene* scene, const float* cameras, uint32_t n_views, const float translation[3], uint32_t scale, uint32_t width,
+                          uint32_t height, int32_t* d_hits_out, float* d_depth_out, uint8_t* d_face_out, uint32_t* d_colour_out);
+
 /* Opt-in L2 residency hint: an access-policy window (persisting) over the structure's hottest array -- the VCS cluster
  * headers or the hash table's slots -- on the handle's current stream (also VRM_L2_PERSIST=1 at vrm_scene_create).  Off by
  * default: on the BASELINE scenes the touched working set already lives in L1/L2 and the window measured no gain. */

@@ -39,6 +39,7 @@ EXPORTS = [
     "vrm_scene_add_dense", "vrm_scene_add_dense_device", "vrm_scene_read_box", "vrm_scene_read_box_device",
     "vrm_scene_read_voxels", "vrm_scene_read_voxels_device",
     "vrm_hit_surface_views", "vrm_hit_surface_views_device", "vrm_hit_surface_rays", "vrm_hit_surface_rays_device",
+    "vrm_cast_rays", "vrm_cast_rays_device", "vrm_cast_views", "vrm_cast_views_device",
 ]
 
 # face codes of the hit surfaces -> outward normal of the face the ray entered through (0 = no hit, then -x, +x, -y, +y, -z, +z)
@@ -117,6 +118,10 @@ def load_library():
         "vrm_hit_surface_views_device": (ci, [vp, vp, u32, vp, u32, u32, u32, vp, vp, vp]),
         "vrm_hit_surface_rays": (ci, [vp, vp, u64, vp, u32, vp, vp, vp]),
         "vrm_hit_surface_rays_device": (ci, [vp, vp, u64, vp, u32, vp, vp, vp]),
+        "vrm_cast_rays": (ci, [vp, vp, vp, u64, vp, u32, vp, vp, vp, vp]),
+        "vrm_cast_rays_device": (ci, [vp, vp, vp, u64, vp, u32, vp, vp, vp, vp]),
+        "vrm_cast_views": (ci, [vp, vp, u32, vp, u32, u32, u32, vp, vp, vp, vp]),
+        "vrm_cast_views_device": (ci, [vp, vp, u32, vp, u32, u32, u32, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -494,6 +499,51 @@ class VoxelScene:
         self._check(self.lib.vrm_hit_surface_rays_device(self.h, C.c_void_p(d_rays_ptr), int(n), _ptr(_f3(translation)), int(scale),
                                                          C.c_void_p(d_hits_ptr), C.c_void_p(d_depth_ptr or 0), C.c_void_p(d_face_ptr or 0)),
                     "vrm_hit_surface_rays_device")
+
+    # -- exact ray casts (include/vrm_b200.h "exact ray casts": first stored voxel along the exact ray within an interval) -----------
+    def cast_rays(self, rays, ranges=None, scale=1, translation=(0.0, 0.0, 0.0)):
+        """The first stored voxel along each exact world ray (n, 6) within its interval ``ranges`` (n, 2) {t_near, t_far} (None: [0, +inf)).
+        Returns dict(hits (n, 4) int32 {x, y, z, 1 | 0}, depth (n,) float32 world ray parameter of the entry (t_near for a hit in the start
+        cell, +inf for a miss), face (n,) uint8 1..6 of the entered face (``FACE_NORMALS``; 0 in the start cell or for a miss),
+        colour (n,) uint32 the stored colour (``EMPTY`` for a miss))."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 6)
+        n = rays.shape[0]
+        rg = None
+        if ranges is not None:
+            rg = np.ascontiguousarray(ranges, np.float32).reshape(-1, 2)
+            if rg.shape[0] != n:
+                raise ValueError(f"ranges holds {rg.shape[0]} intervals for {n} rays")
+        out = dict(hits=np.empty((n, 4), np.int32), depth=np.empty(n, np.float32), face=np.empty(n, np.uint8), colour=np.empty(n, np.uint32))
+        self._check(self.lib.vrm_cast_rays(self.h, _ptr(rays), _ptr(rg), n, _ptr(_f3(translation)), int(scale), _ptr(out["hits"]),
+                                           _ptr(out["depth"]), _ptr(out["face"]), _ptr(out["colour"])), "vrm_cast_rays")
+        return out
+
+    def cast_rays_device(self, d_rays_ptr: int, n: int, d_ranges_ptr: int | None = None, d_hits_ptr: int | None = None, d_depth_ptr: int | None = None,
+                         d_face_ptr: int | None = None, d_colour_ptr: int | None = None, scale=1, translation=(0.0, 0.0, 0.0)):
+        """``cast_rays`` on device buffers (rays, ranges, depth, colour 4-byte aligned, hits 16-byte aligned; each output optional, not all);
+        asynchronous on the scene's stream."""
+        self._check(self.lib.vrm_cast_rays_device(self.h, C.c_void_p(d_rays_ptr), C.c_void_p(d_ranges_ptr or 0), int(n), _ptr(_f3(translation)),
+                                                  int(scale), C.c_void_p(d_hits_ptr or 0), C.c_void_p(d_depth_ptr or 0), C.c_void_p(d_face_ptr or 0),
+                                                  C.c_void_p(d_colour_ptr or 0)), "vrm_cast_rays_device")
+
+    def cast_views(self, cameras, width, height, scale=1, translation=(0.0, 0.0, 0.0)):
+        """``cast_rays`` for the pixel rays of each camera's frame (the render's rays, over [0, +inf)), view-major: hits (n, H, W, 4),
+        depth (n, H, W) = world distance from the camera origin along the pixel's ray, face and colour (n, H, W)."""
+        cams = np.ascontiguousarray(np.stack([self._cam(c) for c in cameras]), np.float32)
+        v = cams.shape[0]
+        out = dict(hits=np.empty((v, height, width, 4), np.int32), depth=np.empty((v, height, width), np.float32),
+                   face=np.empty((v, height, width), np.uint8), colour=np.empty((v, height, width), np.uint32))
+        self._check(self.lib.vrm_cast_views(self.h, _ptr(cams), v, _ptr(_f3(translation)), int(scale), width, height, _ptr(out["hits"]),
+                                            _ptr(out["depth"]), _ptr(out["face"]), _ptr(out["colour"])), "vrm_cast_views")
+        return out
+
+    def cast_views_device(self, cameras, width, height, d_hits_ptr: int | None = None, d_depth_ptr: int | None = None, d_face_ptr: int | None = None,
+                          d_colour_ptr: int | None = None, scale=1, translation=(0.0, 0.0, 0.0)):
+        """``cast_views`` into device buffers (alignment as ``cast_rays_device``); asynchronous on the scene's stream."""
+        cams = np.ascontiguousarray(np.stack([self._cam(c) for c in cameras]), np.float32)
+        self._check(self.lib.vrm_cast_views_device(self.h, _ptr(cams), cams.shape[0], _ptr(_f3(translation)), int(scale), width, height,
+                                                   C.c_void_p(d_hits_ptr or 0), C.c_void_p(d_depth_ptr or 0), C.c_void_p(d_face_ptr or 0),
+                                                   C.c_void_p(d_colour_ptr or 0)), "vrm_cast_views_device")
 
     def lookup(self, xyz):
         xyz = np.ascontiguousarray(xyz, np.int32).reshape(-1, 3)

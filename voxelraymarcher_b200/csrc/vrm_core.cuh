@@ -1393,4 +1393,227 @@ VRM_HD float hit_surface(const int32_t* hit, const float* P, const float* D, con
 	return withLen ? vadd(len, q) : q;
 }
 
+// ---------------------------------------------------------------- exact ray casts (vrm_cast_*, DESIGN.md §3.7)
+//
+// The first STORED voxel along the exact ray within a parameter interval, with its entry depth, face and colour.  The definition is the
+// cell-by-cell walk of include/vrm_b200.h "exact ray casts" in the local frame s = scale * (P - translation), tau = scale * t:
+//   plane k of axis a (D_a != 0) is crossed at tau_a(k) = (k - s_a) / D_a (hit_surface's expression; monotone in k, not strictly once
+//   |k - s_a| passes ~2^23), the walk starts in the cell after every crossing with tau <= tau0 and repeatedly takes the smallest next
+//   crossing, ties to the earlier axis, until it passes tau1.  At one tau the walk therefore makes all of x's crossings, then y's, then
+//   z's, so the walk's state right after axis m crosses a plane at tau X is: axis m in the cell behind that plane, every earlier axis in
+//   the cell after all its crossings <= X, every later axis in the cell after all its crossings < X (cast_search).  That is what makes
+//   the leaps below exact: out of a null 64^3 region, out of an 8^3 cluster whose mask bit is clear, and into the region table's box,
+//   each leap lands in the state the cell-by-cell walk has right after it crosses the exit (entry) plane -- including ties between axes
+//   and runs of equal tau on one axis.  Cells are stepped one by one only inside occupied clusters.
+// This one function is the definition: the sm_100a kernel (vrm_cast.cu) and the CPU tests' host build both call it.
+
+struct CastResult
+{
+	int32_t hit[4];   // global voxel x, y, z and 1; all 0 for a miss
+	float depth;      // world ray parameter (views: distance from the eye); +inf for a miss
+	uint32_t face;    // 1..6 = -x, +x, -y, +y, -z, +z of the entered face; 0 for a hit in the start cell and for a miss
+	uint32_t colour;  // the stored colour (exactly what vrm_lookup returns); kEmpty for a miss
+};
+
+// tau of plane k on one axis, through the ray's exact division (bit-identical to vdiv)
+VRM_HD float cast_tau(int k, float s, float d, float rd, float thr) { return div1(vsub((float)k, s), d, rd, thr); }
+
+// The cell of one axis after every crossing with tau <= X (strict: tau < X), searched in [lo, hi]: the largest m there with
+// P(m) = (d < 0) == (strict ? tau(m) >= X : tau(m) > X), true for every m up to the answer as tau is monotone.  lo - 1 when P fails on
+// all of [lo, hi] (the cell lies below lo); hi when the cell is hi or above.  The first probe is the rounded position s + X d, which
+// is off by at most one cell except in runs of equal tau, so a search usually costs two divisions.
+VRM_HD int cast_search(float s, float d, float rd, float thr, float X, bool strict, int lo, int hi)
+{
+	const bool neg = d < 0.0f;
+	auto P = [&](int m) {
+		const float t = cast_tau(m, s, d, rd, thr);
+		return neg == (strict ? t >= X : t > X);
+	};
+	const float e = vadd(s, vmul(X, d));
+	const int k = e >= (float)hi ? hi : (e >= (float)lo ? (int)floorf(e) : lo);
+	int a = lo - 1, b = hi;  // the answer lies in [a, b]
+	if (P(k)) a = k; else b = k - 1;
+	if (a < b)
+	{
+		const int m = a == k ? k + 1 : k - 1;
+		if (P(m)) a = m; else b = m - 1;
+	}
+	while (a < b)
+	{
+		const int m = a + (b - a + 1) / 2;
+		if (P(m)) a = m; else b = m - 1;
+	}
+	return a;
+}
+
+// The cuckoo lookup with the found flag kept apart from the colour (a voxel may be stored with the colour kEmpty)
+VRM_HD bool cast_hash_probe(const SceneView& sv, const RegionRef<kStorageHash>& r, uint32_t key, uint32_t& colour)
+{
+	const unsigned long long e1 = ldg(sv.slots + (r.base1 + hash_slot1(key, r.seed1, r.n)));
+	const unsigned long long e2 = ldg(sv.slots + (r.base2 + hash_slot2(key, r.seed2, r.n)));
+	if (slot_key(e1) == key) { colour = slot_colour(e1); return true; }
+	if (slot_key(e2) == key) { colour = slot_colour(e2); return true; }
+	return false;
+}
+
+// One ray.  P, D: world origin and direction; [tNear, tFar]: the interval of the world ray parameter.  withLen (views): depth = len +
+// tau / scale, len for a start-cell hit; otherwise depth = tau / scale, tNear for a start-cell hit.
+template <int ST>
+VRM_HD void cast_ray(const SceneView& sv, const float* P, const float* D, const float* tr, float scale, float tNear, float tFar, float len,
+                     bool withLen, CastResult& res)
+{
+	res.hit[0] = res.hit[1] = res.hit[2] = res.hit[3] = 0;
+	res.depth = INFINITY; res.face = 0u; res.colour = kEmpty;
+	if (!(isfinite(P[0]) && isfinite(P[1]) && isfinite(P[2]) && isfinite(D[0]) && isfinite(D[1]) && isfinite(D[2]) && isfinite(tNear)) ||
+	    tFar != tFar || tNear > tFar)
+		return;
+	float s[3];
+	for (int a = 0; a < 3; a++) s[a] = vmul(scale, vsub(P[a], tr[a]));
+	const float tau0 = vmul(tNear, scale), tau1 = vmul(tFar, scale);
+	// an overflowing local origin or start (huge coordinates, a non-finite translation) has no cell: a miss
+	if (!(isfinite(s[0]) && isfinite(s[1]) && isfinite(s[2]) && isfinite(tau0))) return;
+	RayDir k = make_raydir(D[0], D[1], D[2]);
+	// the fast division also needs its quotients far from overflow: |k - s| < 2^65, |q| < 2^105
+	if (!(fabsf(s[0]) < 1.8446744e19f && fabsf(s[1]) < 1.8446744e19f && fabsf(s[2]) < 1.8446744e19f)) k.thr = NAN;
+	const int L = kRegion * sv.minCoord, Hb = L + kRegion * (int)sv.diameter;  // the region table's box [L, Hb)^3
+	auto tau = [&](int a, int plane) { return cast_tau(plane, s[a], k.d[a], k.rd[a], k.thr); };
+	auto next = [&](int a, int cell) { return tau(a, k.d[a] > 0.0f ? cell + 1 : cell); };  // the next crossing out of `cell`
+	auto search = [&](int a, float X, bool strict, int lo, int hi) { return cast_search(s[a], k.d[a], k.rd[a], k.thr, X, strict, lo, hi); };
+	auto inBox = [&](int v) { return v >= L && v < Hb; };
+
+	// start cell: the cell after every crossing with tau <= tau0 (searched in [L - 1, Hb]: only its cell inside the box matters)
+	int c[3];
+	for (int a = 0; a < 3; a++)
+	{
+		if (k.d[a] == 0.0f)
+		{
+			const float fl = floorf(s[a]);
+			if (!(fl >= (float)L && fl < (float)Hb)) return;  // the axis never moves: the ray never enters the box
+			c[a] = (int)fl;
+		}
+		else c[a] = search(a, tau0, false, L - 1, Hb);
+	}
+	float t = tau0;
+	uint32_t face = 0u;
+	if (!(inBox(c[0]) && inBox(c[1]) && inBox(c[2])))
+	{
+		// leap to the box: its entry is the latest per-axis entry crossing (ties: the later axis crosses last)
+		int m = -1;
+		float E = 0.0f;
+		for (int a = 0; a < 3; a++)
+		{
+			if (k.d[a] == 0.0f || inBox(c[a])) continue;
+			if ((c[a] < L) != (k.d[a] > 0.0f)) return;  // outside and moving away
+			const float Ea = tau(a, c[a] < L ? L : Hb);
+			if (m < 0 || Ea >= E) { E = Ea; m = a; }
+		}
+		if (!(E <= tau1)) return;
+		for (int b = 0; b < 3; b++)
+		{
+			if (b == m || k.d[b] == 0.0f) continue;
+			c[b] = search(b, E, b > m, L - 1, Hb);
+			if (!inBox(c[b])) return;  // another axis left the box before this one entered it
+		}
+		c[m] = k.d[m] > 0.0f ? L : Hb - 1;
+		t = E;
+		face = 1u + 2u * (uint32_t)m + (k.d[m] < 0.0f ? 1u : 0u);
+	}
+	float nt[3];
+	for (int a = 0; a < 3; a++) nt[a] = k.d[a] != 0.0f ? next(a, c[a]) : 0.0f;
+
+	// Leap to the exit of the aligned cube of side S around c: the first exit crossing (ties: the earlier axis), the crossing axis into
+	// the cell behind it, the others by cast_search inside the cube.  false: the walk ends (past tau1, no moving axis, out of the box).
+	auto leap = [&](int S) -> bool {
+		int m = -1;
+		float X = 0.0f;
+		for (int a = 0; a < 3; a++)
+		{
+			if (k.d[a] == 0.0f) continue;
+			const int lo = c[a] & -S;
+			const float Xa = tau(a, k.d[a] > 0.0f ? lo + S : lo);
+			if (m < 0 || Xa < X) { X = Xa; m = a; }
+		}
+		if (m < 0 || !(X <= tau1)) return false;
+		for (int b = 0; b < 3; b++)
+		{
+			if (b == m || k.d[b] == 0.0f) continue;
+			const int lo = c[b] & -S;
+			c[b] = search(b, X, b > m, lo, lo + S - 1);
+			nt[b] = next(b, c[b]);
+		}
+		c[m] = k.d[m] > 0.0f ? (c[m] & -S) + S : (c[m] & -S) - 1;
+		nt[m] = next(m, c[m]);
+		t = X;
+		face = 1u + 2u * (uint32_t)m + (k.d[m] < 0.0f ? 1u : 0u);
+		return inBox(c[m]);
+	};
+	// One crossing of the cell-by-cell walk.  false: the walk ends.
+	auto step = [&]() -> bool {
+		int m = -1;
+		for (int a = 0; a < 3; a++)
+			if (k.d[a] != 0.0f && (m < 0 || nt[a] < nt[m])) m = a;
+		if (m < 0 || !(nt[m] <= tau1)) return false;
+		t = nt[m];
+		face = 1u + 2u * (uint32_t)m + (k.d[m] < 0.0f ? 1u : 0u);
+		c[m] += k.d[m] > 0.0f ? 1 : -1;
+		nt[m] = next(m, c[m]);
+		return inBox(c[m]);
+	};
+
+	const uint32_t Dm = sv.diameter;
+	for (;;)  // regions
+	{
+		const uint32_t u0 = (uint32_t)(c[0] - L) >> 6, u1 = (uint32_t)(c[1] - L) >> 6, u2 = (uint32_t)(c[2] - L) >> 6;
+		const int32_t ri = ldg(sv.regionTable + (u0 + u1 * Dm + u2 * Dm * Dm));
+		if (ri < 0)
+		{
+			if (!leap(kRegion)) return;
+			continue;
+		}
+		const RegionRef<ST> r = load_region<ST>(sv, ri);
+		const int rg0 = c[0] & -kRegion, rg1 = c[1] & -kRegion, rg2 = c[2] & -kRegion;
+		auto inRegion = [&]() { return (c[0] & -kRegion) == rg0 && (c[1] & -kRegion) == rg1 && (c[2] & -kRegion) == rg2; };
+		for (;;)  // clusters of the region
+		{
+			const uint32_t cid = vcs_cluster_id((uint32_t)(c[0] - rg0) >> 3, (uint32_t)(c[1] - rg1) >> 3, (uint32_t)(c[2] - rg2) >> 3);
+			if (!((ldg(sv.clusterMask + (r.ri * 16u + (cid >> 5))) >> (cid & 31u)) & 1u))
+			{
+				if (!leap(8)) return;
+				if (!inRegion()) break;
+				continue;
+			}
+			const int cl0 = c[0] & -8, cl1 = c[1] & -8, cl2 = c[2] & -8;
+			uint32_t wordAt = 0xFFFFFFFFu;  // VCS: the header word in hand (32 cells' occupancy)
+			uint2 h = {0u, 0u};
+			for (;;)  // cells of the cluster
+			{
+				const uint32_t x = (uint32_t)(c[0] - rg0), y = (uint32_t)(c[1] - rg1), z = (uint32_t)(c[2] - rg2);
+				bool found;
+				uint32_t colour = kEmpty;
+				if constexpr (ST == kStorageVcs)
+				{
+					const uint32_t code = ((x & 7u) << 6) | ((y & 7u) << 3) | (z & 7u);
+					if (code >> 5 != wordAt) { wordAt = code >> 5; h = ldg(sv.headers + vcs_header_index(r.ri, cid, wordAt)); }
+					const uint32_t bit = code & 31u;
+					found = (h.x >> bit) & 1u;
+					if (found) colour = ldg(sv.values + vcs_colour_index(h.x, h.y, bit));
+				}
+				else found = cast_hash_probe(sv, r, hash_key(x, y, z), colour);
+				if (found)
+				{
+					res.hit[0] = c[0]; res.hit[1] = c[1]; res.hit[2] = c[2]; res.hit[3] = 1;
+					res.face = face;
+					res.colour = colour;
+					if (face == 0u) res.depth = withLen ? len : tNear;
+					else { const float q = vdiv(t, scale); res.depth = withLen ? vadd(len, q) : q; }
+					return;
+				}
+				if (!step()) return;
+				if ((c[0] & -8) != cl0 || (c[1] & -8) != cl1 || (c[2] & -8) != cl2) break;
+			}
+			if (!inRegion()) break;
+		}
+	}
+}
+
 }  // namespace vrm
