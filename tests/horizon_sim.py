@@ -87,11 +87,11 @@ class Scene:
             self.lib.sim_scene_destroy(self.h)
             self.h = None
 
-    def render(self, cam, w, h, algorithm, scale=1, horizon=True, threads=None):
+    def render(self, cam, w, h, algorithm, scale=1, horizon=True, threads=None, translation=(0.0, 0.0, 0.0)):
         rgb = np.zeros((h, w, 3), np.uint8)
         hits = np.zeros((h, w, 4), np.int32)
         counters = np.zeros(5, np.uint64)
-        rc = self.lib.hz_render(self.h, _p(np.ascontiguousarray(cam, np.float32)), _p(_f3((0, 0, 0))), scale, ALGORITHM[algorithm], w, h,
+        rc = self.lib.hz_render(self.h, _p(np.ascontiguousarray(cam, np.float32)), _p(_f3(translation)), scale, ALGORITHM[algorithm], w, h,
                                 _p(rgb), _p(hits), _p(counters), threads or (os.cpu_count() or 1), int(horizon))
         assert rc == 0, rc
         return dict(rgb=rgb, hits=hits, counters=counters)

@@ -232,4 +232,48 @@ int hz_property(void* h, const float* rays, uint64_t n, int algorithm, uint64_t*
 	return 0;
 }
 
+// The threshold of shadow rays started at hit points (hitW region-local, regW their regions; WORLD axes, scale 1) of the longest-axis kind
+// (la != 0) or the original one, with the scene's map for gLight -- or every cell set to cellValue (override != 0).  out: computed = the
+// unclamped ceilf value (NaN when the threshold axis has n_a = 0), thr = horizon_threshold(), word = the threshold start_shadow left in
+// the flag word.  Returns 1 when the light gets no map.
+int hz_threshold_check(void* h, const float* hitW, const int32_t* regW, uint64_t n, int la, int override, int32_t cellValue, float* computed,
+                       int32_t* thr, int32_t* word)
+{
+	SimScene* s = static_cast<SimScene*>(h);
+	if (s->storage != kStorageVcs) return 2;
+	std::vector<int32_t> cells;
+	const HorizonView hv = horizon_map(*s, cells);
+	if (!hv.cells) return 1;
+	if (override) std::fill(cells.begin(), cells.end(), cellValue);
+	RayCtx<kStorageVcs, true> c;
+	c.sv = s->view(); c.light = gLight; c.lw = make_light_walk(gLight); c.hitOut = nullptr; c.hv = hv;
+	c.translation[0] = c.translation[1] = c.translation[2] = 0.0f;
+	for (uint64_t i = 0; i < n; i++)
+	{
+		c.reset();
+		c.hv = hv;
+		ShadowStart ss;
+		for (int a = 0; a < 3; a++) { ss.hitW[a] = hitW[3 * i + a]; ss.regW[a] = regW[3 * i + a]; }
+		ss.lit = 0xFFFFFFu;
+		ss.la = la ? 1 : 0;
+		FlatRay<kStorageVcs, kAlgoLongestAxis, true> ray;
+		ray.start_shadow(c, ss);
+		word[i] = (int32_t)ray.fl >> kFlHzShift;
+		thr[i] = ray.horizon_threshold(c, ss);
+		// horizon_threshold's arithmetic before its clamp
+		float pw[3];
+		for (int a = 0; a < 3; a++) pw[a] = (float)((ss.regW[a] - c.sv.minCoord) * kRegion) + ss.hitW[a];
+		int iu = (int)floorf((pw[0] * hv.e1[0] + pw[1] * hv.e1[1] + pw[2] * hv.e1[2] - hv.u0) * hv.invCell);
+		int iv = (int)floorf((pw[0] * hv.e2[0] + pw[1] * hv.e2[1] + pw[2] * hv.e2[2] - hv.v0) * hv.invCell);
+		iu = iu < 0 ? 0 : (iu >= (int)hv.nu ? (int)hv.nu - 1 : iu);
+		iv = iv < 0 ? 0 : (iv >= (int)hv.nv ? (int)hv.nv - 1 : iv);
+		const int32_t top = hv.cells[(uint32_t)iv * hv.nu + (uint32_t)iu];
+		const float depth0 = pw[0] * hv.n[0] + pw[1] * hv.n[1] + pw[2] * hv.n[2];
+		const int ax = la ? hv.axis : 0;
+		const float na = hv.n[ax], pa = pw[ax];
+		computed[i] = na == 0.0f ? NAN : ceilf((na < 0.0f ? -pa : pa) + ((float)top + kHorizonMargin - depth0) * fabsf(na));
+	}
+	return 0;
+}
+
 }  // extern "C"
